@@ -1,24 +1,30 @@
 #!/usr/bin/env python
 """bench.py -- M^-1 applies/s of the multilevel HIF preconditioner on B200 (BASELINE.json metric).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
-Workload (configs[1]): synthetic 3D Poisson 7-point 128^3 (n = 2 097 152), HIF factorized on the
-host by the unmodified reference with its PDE parameter set, nrhs = 1.  One "step" = one M^-1
-apply (hif::HIF::solve) of a seeded right-hand side.
+Workload (configs[1]): synthetic 3D Poisson 7-point 128^3 (n = 2 097 152), nrhs = 1.  One "step"
+= one M^-1 apply (hif::HIF::solve semantics) of a seeded right-hand side.
 
   value : applies/s with b and x resident in HBM (lhfdGpuSolveDev), whole job over all ranks
   e2e   : applies/s through lhfdGpuSolve with pinned HOST b/x (H2D + apply + D2H per step)
   roofline : algorithmic bytes per apply (SURVEY.md 8d) / measured time vs measured HBM copy peak
-  cpu_baseline : the reference's own hif::HIF::solve on this box's host, 1 core (it is serial)
+  cpu_baseline : the C restatement of the reference's serial apply (oracle/hif_oracle.c), 1 core
 
 Multi-GPU: the apply does not shard (sequential levels); every rank holds a factor replica and
 applies to its own right-hand sides -> weak scaling, no collective on the hot path; results are
 gathered with one NCCL all_gather after the timed region.
 
-The factorization (host, reference code) is the factor PRODUCER the device backend attaches to;
-it runs before the timed region and is never part of a reported number.
+Factors: multilevel HIF factors computed on the host by oracle/factor.py (scaling, permutations, D-ILU
+leading blocks, E/F blocks, sparse Schur levels, dense QRCP last level), so that the benchmark needs
+nothing outside the repository.  The factorization runs before the timed region and is never part of a
+reported number; the parity check before timing compares with the C oracle on the same factors.
+
+--dump-outputs DIR writes what the timed path returned in its last step as DIR/<name>.npy (float64;
+a fixed seeded sample of rows when the whole would exceed 64 MB), so that two builds can be compared
+output for output: the inputs depend only on the arguments.  Both arms apply step k to right-hand
+side k % NB_RHS, so their dumps are solutions of the same system.
 """
 import argparse
 import json
@@ -54,29 +60,49 @@ def workload_name(workload, size, nrhs):
     return f"{workload} {shape} nrhs={nrhs}"
 
 
-def factorize(A, threads, nsp=False, dtype=np.float64):
-    """Host factorization by the unmodified reference (factor producer + CPU oracle).
-    dtype=float32: hif::HIF<float,int> factorized from the double matrix (mixed precision)."""
-    from hifir_b200 import problems as P
-    from oracle import refhost as R
+FACTORS = "multilevel D-ILU, independent-set Schur levels, dense QRCP last level (oracle/factor.py)"
+
+
+class HostFactor:
+    """Factors for the device backend plus the C oracle applied to the same factors (parity check and
+    CPU baseline): solve / hifir / krylov / set_nsp_const are those of oracle.port.OracleHif."""
+
+    def __init__(self, A, levels):
+        from oracle import port as O
+        self._levels = levels
+        self.oracle = O.OracleHif(levels, A)
+        self.nnz = sum(len(L[k][3]) for L in levels for k in "LUEF")
+
+    def levels(self):
+        return self._levels
+
+    def __getattr__(self, name):
+        return getattr(self.oracle, name)
+
+
+def factorize(A, nsp=False, dtype=np.float64):
+    """Host factorization (oracle/factor.py), wrapped with the C oracle on the same factors.
+    dtype=float32: single-precision factors of the double matrix (lhfs* / lhfsd* entry points)."""
+    from oracle import factor as F
     t0 = time.time()
-    M = R.RefHif(A, P.PDE_PARAMS, threads=threads, dtype=dtype)
+    M = HostFactor(A, F.multilevel_levels(A, dtype))
     if nsp:
         M.set_nsp_const()
-    log(f"[bench] reference factorize: {time.time() - t0:.1f} s, levels {M.num_levels}, nnz {M.nnz}")
+    log(f"[bench] factorize: {time.time() - t0:.1f} s, levels {len(M.levels())}, nnz {M.nnz}")
     return M
 
 
-def cached_levels(workload, size, threads=None):
-    """Per-level factors for developer tools: reference factorization, cached on local disk
-    (uncompressed npz) so that several processes on one box factorize once."""
+def cached_levels(workload, size):
+    """Per-level factors for developer tools: factorize(), cached on local disk (uncompressed npz)
+    so that several processes on one box factorize once; the key names the factor producer."""
     from hifir_b200.levels_io import arrays_to_levels, levels_to_arrays
-    path = os.path.join(CACHE_DIR, f"{workload}{size}.npz")
+    from oracle import factor as F
+    path = os.path.join(CACHE_DIR, f"{workload}{size}_{F.NAME_KEY}.npz")
     A = make_problem(workload, size)
     if os.path.exists(path):
         with np.load(path) as z:
             return A, arrays_to_levels({k: z[k] for k in z.files})
-    M = factorize(A, threads=threads or os.cpu_count() or 1)
+    M = factorize(A)
     levels = M.levels()
     os.makedirs(CACHE_DIR, exist_ok=True)
     np.savez(path, **levels_to_arrays(levels))
@@ -141,19 +167,22 @@ def hbm_peak():
 
 
 # ----------------------------------------------------------------------------- reference arm
+NB_RHS = 4  # step k of either arm applies to right-hand side k % NB_RHS
+
+
 def cpu_apply_rate(M, n, applies, warm=1, nirs=1, A=None):
-    """nirs > 1: a step is one hif::HIF::hifir(A, b, nirs, x) (builder.hpp:458-465) = nirs applies;
-    the right-hand sides are then consistent (b = A v), as config 5 asks."""
-    from hifir_b200 import problems as P
-    bs = [step_rhs(A, n, j, nirs) for j in range(2)]
+    """The C oracle's apply; nirs > 1: a step is one hifir(A, b, nirs, x) = nirs applies (the
+    right-hand sides are then consistent, b = A v, as config 5 asks).  Returns (rate, seconds, x of the
+    last step)."""
+    bs = [step_rhs(A, n, j, nirs) for j in range(NB_RHS)]
     f = (lambda b: M.solve(b)) if nirs <= 1 else (lambda b: M.hifir(b, nirs))
     for _ in range(warm):
         f(bs[0])
     t0 = time.perf_counter()
     for k in range(applies):
-        f(bs[k % 2])
+        x = f(bs[k % NB_RHS])
     dt = time.perf_counter() - t0
-    return applies / dt, dt
+    return applies / dt, dt, x
 
 
 def step_rhs(A, n, j, nirs):
@@ -165,14 +194,13 @@ def step_rhs(A, n, j, nirs):
     return P.csr_matvec(A, np.sin(0.37 * np.arange(n) + j))
 
 
-def _ref_batched_worker(wid, T, workload, size, nrhs, steps, threads, ready, go, out):
-    """One reference object per worker: hif::HIF is neither copyable (Prec.hpp:134) nor re-entrant
-    (mutable work buffer, builder.hpp:579), so a throughput baseline over independent columns needs T
-    factorized objects (SURVEY.md 8d)."""
+def _ref_batched_worker(wid, T, workload, size, nrhs, steps, ready, go, out):
+    """One process of the batched CPU arm: factorizes, then applies the C oracle to its columns
+    wid, wid + T, ... of the block, `steps` times (the oracle, like hif::HIF, applies one column at a time
+    on one thread)."""
     from hifir_b200 import problems as P
-    os.environ["OMP_NUM_THREADS"] = str(threads)
     A = make_problem(workload, size)
-    M = factorize(A, threads=threads)
+    M = factorize(A)
     cols = list(range(wid, nrhs, T))  # this worker's columns of the block
     B = P.seeded_rhs(A[0], 0, nrhs=nrhs)
     bs = [np.ascontiguousarray(B[:, k]) for k in cols]
@@ -188,21 +216,18 @@ def _ref_batched_worker(wid, T, workload, size, nrhs, steps, threads, ready, go,
 
 
 def run_reference_batched(args):
-    """--impl reference --nrhs K: the reference's batched apply is a column loop of hif::HIF::solve (its own
-    multi-rhs driver is defective, SURVEY.md App. B-1); with all the host threads it can use that is T
-    objects applying disjoint columns concurrently."""
+    """--impl reference --nrhs K: a batched CPU apply is a column loop of single solves (the reference's own
+    multi-rhs driver is defective, SURVEY.md App. B-1); T processes apply disjoint columns concurrently."""
     import multiprocessing as mp
     nproc = os.cpu_count() or 1
     T = max(1, min(nproc, 8, args.nrhs))
-    threads = max(1, nproc // T)
     A = make_problem(args.workload, args.size)
     n = A[0]
-    # a step = one block of nrhs columns; bounded sample of steps (~0.07 s per column at 96^3)
-    steps = max(1, min(args.steps, args.ref_max_steps // max(1, -(-args.nrhs // T)) // 4 or 1))
+    steps = args.steps  # a step = one block of nrhs columns
     ctx = mp.get_context("spawn")
     ready, out, go = ctx.Queue(), ctx.Queue(), ctx.Event()
     ws = [ctx.Process(target=_ref_batched_worker,
-                      args=(w, T, args.workload, args.size, args.nrhs, steps, threads, ready, go, out)) for w in range(T)]
+                      args=(w, T, args.workload, args.size, args.nrhs, steps, ready, go, out)) for w in range(T)]
     for w in ws:
         w.start()
     for _ in ws:
@@ -214,16 +239,15 @@ def run_reference_batched(args):
     cols = sum(r[1] for r in res)
     wall = max(r[3] for r in res) - min(r[2] for r in res)
     rate = cols / wall
-    sample = (f"{steps} of the {args.steps} requested blocks of {args.nrhs} columns: {T} factorized hif::HIF objects "
-              f"(one per process, {threads} OpenMP thread(s) each for the factorization), each applying its "
-              f"{-(-args.nrhs // T)} columns of the block with hif::HIF::solve; {cols} applies in {wall:.1f} s")
+    sample = (f"{steps} blocks of {args.nrhs} columns: {T} processes, each applying its "
+              f"{-(-args.nrhs // T)} columns of the block with the C oracle's solve; {cols} applies in {wall:.1f} s")
     line = {
         "impl": "reference", "metric": "M^-1 applies/sec", "value": rate, "unit": "applies/s", "n_gpus": args.gpus,
         "steps": steps, "warmup": args.warmup, "ms_per_step": 1e3 * wall / steps, "higher_is_better": True,
         "scaling": "strong", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
         "config": {"workload": workload_name(args.workload, args.size, args.nrhs), "n": n,
-                   "params": "tau=1e-2 alpha=3 kappa=5 (reference PDE set)", "l2_policy": L2_POLICY},
-        "cpu_baseline": {"value": rate, "unit": "applies/s", "cores": T, "kind": "reference", "sample": sample},
+                   "params": FACTORS, "l2_policy": L2_POLICY},
+        "cpu_baseline": {"value": rate, "unit": "applies/s", "cores": T, "kind": "oracle", "sample": sample},
         "e2e": {"value": rate, "unit": "applies/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
     }
@@ -239,27 +263,27 @@ def run_reference(args, rank, world):
     n = A[0]
     single = args.precision == "single"
     nirs = args.nirs
-    M = factorize(A, threads=os.cpu_count() or 1, nsp=args.workload == "neumann",
+    M = factorize(A, nsp=args.workload == "neumann",
                   dtype=np.float32 if single else np.float64)
-    steps = min(args.steps, max(1, args.ref_max_steps // nirs))
+    steps = args.steps
     cpu_apply_rate(M, n, max(1, min(args.warmup, 3)), warm=0, nirs=nirs, A=A)
-    rate, dt = cpu_apply_rate(M, n, steps, warm=0, nirs=nirs, A=A)
+    rate, dt, x = cpu_apply_rate(M, n, steps, warm=0, nirs=nirs, A=A)
     rate *= nirs  # applies/s: a refinement step holds nirs applies
-    sample = (f"{steps} of the {args.steps} requested hif::HIF::solve applies (serial reference code, "
-              f"prec_solve.hpp:332-412 has no threading), each a full apply of the workload") if nirs <= 1 else (
-              f"{steps} of the {args.steps} requested hif::HIF::hifir(A, b, nirs={nirs}) solves = {steps * nirs} applies "
-              f"+ {steps * (nirs - 1)} A x (OpenMP, {os.cpu_count()} threads); the apply itself is serial")
+    sample = (f"{steps} serial applies of the C oracle, each a full apply of the workload") if nirs <= 1 else (
+              f"{steps} hifir(A, b, nirs={nirs}) solves of the C oracle = {steps * nirs} applies + {steps * (nirs - 1)} A x")
     line = {
         "impl": "reference", "metric": "M^-1 applies/sec", "value": rate, "unit": "applies/s", "n_gpus": args.gpus,
         "steps": steps, "warmup": args.warmup, "ms_per_step": 1e3 * dt / steps, "higher_is_better": True,
         "scaling": "weak", "vs_baseline": None, "dtype": "f32" if single else "f64", "data": "synthetic",
         "config": {"workload": workload_name(args.workload, args.size, args.nrhs) + (" single-precision factors" if single else "")
                    + (f" hifir nirs={nirs}" if nirs > 1 else ""),
-                   "n": n, "params": "tau=1e-2 alpha=3 kappa=5 (reference PDE set)", "l2_policy": L2_POLICY},
-        "cpu_baseline": {"value": rate, "unit": "applies/s", "cores": 1, "kind": "reference", "sample": sample},
+                   "n": n, "params": FACTORS, "l2_policy": L2_POLICY},
+        "cpu_baseline": {"value": rate, "unit": "applies/s", "cores": 1, "kind": "oracle", "sample": sample},
         "e2e": {"value": rate, "unit": "applies/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, x=x)
     print(json.dumps(line), flush=True)
 
 
@@ -291,7 +315,7 @@ def run_mrhs(args, rank, world, local_rank):
     build.build()
     A = make_problem(args.workload, args.size)
     n, nrhs = A[0], args.nrhs
-    M = factorize(A, threads=max(1, (os.cpu_count() or 1) // world))
+    M = factorize(A)
     levels = M.levels()
     G = hb.GpuHif(levels, device=local_rank)
     st = G.stats()
@@ -363,9 +387,10 @@ def run_mrhs(args, rank, world, local_rank):
         for k in range(ncols):
             M.solve(np.ascontiguousarray(B[:, k]))
         dt = time.perf_counter() - t0
-        cpu = {"value": ncols / dt, "unit": "applies/s", "cores": 1, "kind": "reference",
-               "sample": f"{ncols} of the {nrhs} columns, one hif::HIF::solve each on the same factorized object "
-                         f"({dt:.1f} s; serial reference code, one object = one thread, builder.hpp:579)"}
+        cpu = {"value": ncols / dt, "unit": "applies/s", "cores": 1, "kind": "oracle",
+               "sample": f"{ncols} of the {nrhs} columns, one serial C oracle solve each on the same factors ({dt:.1f} s)"}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, X=X.cpu().numpy())
     nloc0 = max(1, shard_range(nrhs, world, 0)[1])
     width = 64 if nloc0 >= 64 else 32 if nloc0 > 16 else 16 if nloc0 > 8 else 8  # mrhs.cu: apply_mrhs_dev
     chunks = -(-nloc0 // width)
@@ -375,7 +400,7 @@ def run_mrhs(args, rank, world, local_rank):
         "n_gpus": world, "steps": args.steps, "warmup": args.warmup, "ms_per_step": ms_step, "higher_is_better": True,
         "scaling": "strong", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
         "config": {"workload": workload_name(args.workload, args.size, nrhs), "n": n, "levels": st["levels"],
-                   "nnz_factors": st["nnz"], "params": "tau=1e-2 alpha=3 kappa=5 (reference PDE set)",
+                   "nnz_factors": st["nnz"], "params": FACTORS,
                    "l2_policy": "inputs larger than L2",
                    "parallelism": f"replicas, {nrhs} columns sharded over {world} GPU(s), {width} columns per pass"},
         "roofline": {"bound": "hbm", "kernel": "whole batched apply", "achieved": bytes_step / (ms_step * 1e-3) / 1e9,
@@ -386,10 +411,26 @@ def run_mrhs(args, rank, world, local_rank):
         "e2e": {"value": nrhs * args.steps / (e2e_ms * 1e-3), "unit": "applies/s",
                 "h2d_bytes_per_step": 8 * n * nrhs, "d2h_bytes_per_step": 8 * n * nrhs,
                 "api": "lhfdGpuSolveMrhs (pinned host buffers)"},
-        "gpu_launches": launches, "clocks": clocks, "parity_vs_reference": parity,
+        "gpu_launches": launches, "clocks": clocks, "parity_vs_oracle": parity,
         "gathered_shape": list(X.shape),
     }
     print(json.dumps(line), flush=True)
+
+
+DUMP_BYTES = 63 << 20  # array data of --dump-outputs: the .npy headers stay inside 64 MB
+
+
+def dump_outputs(path, **arrays):
+    """Write each array as path/<name>.npy in float64.  When all of them together exceed DUMP_BYTES,
+    each is replaced by a fixed, seeded, sorted sample of its rows."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_BYTES:
+            keep = max(1, len(a) * DUMP_BYTES // total)
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def pin_to_gpu_numa(local_rank):
@@ -427,7 +468,7 @@ def pin_to_gpu_numa(local_rank):
 
 # timing rule of the contract (the same words in both arms' `config`): no L2 flush between steps because one
 # step streams far more than the cache holds
-L2_POLICY = "inputs larger than L2: the factors one apply streams (0.4-1.3 GB) exceed the 126 MB L2, no flush between steps"
+L2_POLICY = "inputs larger than L2: the factors one apply streams exceed the 126 MB L2 at 128^3, no flush between steps"
 REPEATS = 5  # timed repeats of the --steps steps; the median is reported (SURVEY.md 8d)
 
 
@@ -470,12 +511,11 @@ def extra_workload(kind, args, rank, world, local_rank, barrier, stream):
     if args.extras_small:
         size = {"mrhs": 24, "hifir": 24, "stokes": 48}[kind]
     steps = max(2, min(args.steps, args.extra_steps))
-    threads = max(1, (os.cpu_count() or 1) // world)
     A = make_problem(wl, size)
     n = A[0]
     nsp = wl == "neumann"
     t0 = time.time()
-    M = factorize(A, threads=threads, nsp=nsp)
+    M = factorize(A, nsp=nsp)
     t_fact = time.time() - t0
     G = hb.GpuHif(M.levels(), device=local_rank)
     G.set_stream(stream.cuda_stream)
@@ -500,7 +540,7 @@ def extra_workload(kind, args, rank, world, local_rank, barrier, stream):
                 xr = M.solve(np.ascontiguousarray(B[:, b0 + c]))
                 errs.append(float(np.linalg.norm(Xd[:, c].cpu().numpy() - xr) / np.linalg.norm(xr)))
             ms = timed_repeats(lambda k: G.solve_mrhs_dev(nloc, Bd.data_ptr(), Xd.data_ptr(), 0), steps, barrier, stream, 3)
-            rec.update(parity_vs_reference=max(errs), local_ms=ms, nrhs=nrhs, local_columns=nloc,
+            rec.update(parity_vs_oracle=max(errs), local_ms=ms, nrhs=nrhs, local_columns=nloc,
                        bytes_per_block=world * (st["bytes_factors"] + st["bytes_dense"]) + nrhs * st["bytes_vec_per_rhs"])
         elif kind == "hifir":
             G.set_matrix(A)
@@ -513,7 +553,7 @@ def extra_workload(kind, args, rank, world, local_rank, barrier, stream):
             xr = M.hifir(bh, nirs)
             err = float(np.linalg.norm(xd.cpu().numpy() - xr) / np.linalg.norm(xr))
             ms = timed_repeats(lambda k: G.hifir_dev(bd.data_ptr(), nirs, xd.data_ptr()), steps, barrier, stream, 3)
-            rec.update(parity_vs_reference=err, local_ms=ms, nirs=nirs)
+            rec.update(parity_vs_oracle=err, local_ms=ms, nirs=nirs)
         else:
             bh = P.seeded_rhs(n, rank)
             bd = torch.from_numpy(bh).cuda()
@@ -523,7 +563,7 @@ def extra_workload(kind, args, rank, world, local_rank, barrier, stream):
             xr = M.solve(bh)
             err = float(np.linalg.norm(xd.cpu().numpy() - xr) / np.linalg.norm(xr))
             ms = timed_repeats(lambda k: G.solve_dev(bd.data_ptr(), xd.data_ptr(), 0), steps, barrier, stream, 3)
-            rec.update(parity_vs_reference=err, local_ms=ms, depths=G.depths().tolist(),
+            rec.update(parity_vs_oracle=err, local_ms=ms, depths=G.depths().tolist(),
                        bytes_per_apply=st["bytes_factors"] + st["bytes_dense"] + st["bytes_vec_per_rhs"])
         G.synchronize()
     finally:
@@ -545,10 +585,9 @@ def run_ours(args, rank, world, local_rank):
     A = make_problem(args.workload, args.size)
     n = A[0]
     nsp = args.workload == "neumann"
-    threads = max(1, (os.cpu_count() or 1) // world)
     single = args.precision == "single"
     t0 = time.time()
-    M = factorize(A, threads=threads, nsp=nsp, dtype=np.float32 if single else np.float64)
+    M = factorize(A, nsp=nsp, dtype=np.float32 if single else np.float64)
     t_fact = time.time() - t0
     levels = M.levels()
     t0 = time.time()
@@ -565,7 +604,7 @@ def run_ours(args, rank, world, local_rank):
     torch.cuda.set_stream(stream)
     G.set_stream(stream.cuda_stream)
 
-    nb = 4
+    nb = NB_RHS
     nirs = args.nirs  # > 1: a step is one hifir(A, b, nirs, x) = nirs applies + nirs - 1 residuals (config 5)
     b_host = [torch.from_numpy(step_rhs(A, n, rank * nb + j, nirs)).pin_memory() for j in range(nb)]
     b_dev = [b.cuda() for b in b_host]
@@ -593,12 +632,12 @@ def run_ours(args, rank, world, local_rank):
         else:
             x_host[0].numpy()[:] = G.apply(b_host[k % nb].numpy(), nirs=nirs)[0]
 
-    # ---- parity spot check before timing (against the reference's own apply, same object)
+    # ---- parity spot check before timing (against the C oracle's apply of the same factors)
     step_dev(0)
     G.synchronize()
     xr = M.solve(b_host[0].numpy()) if nirs <= 1 else M.hifir(b_host[0].numpy(), nirs)
     parity = float(np.linalg.norm(x_dev.cpu().numpy() - xr) / np.linalg.norm(xr))
-    log(f"[bench] rank {rank}: parity vs reference apply = {parity:.2e}")
+    log(f"[bench] rank {rank}: parity vs oracle apply = {parity:.2e}")
     gate = 1e-5 if single else 1e-12  # north_star tolerances (float / double)
     assert parity <= gate, f"parity gate failed: {parity}"
 
@@ -639,6 +678,11 @@ def run_ours(args, rank, world, local_rank):
         # result gather, off the timed path (the only NCCL traffic of this benchmark)
         out = [torch.empty_like(x_dev) for _ in range(world)]
         dist.all_gather(out, x_dev)
+    # x_dev still holds the last timed step's result (the host-buffer steps use their own buffers); later
+    # calls reuse it.  With several ranks: one row per rank, the gathered result.
+    x_last = None
+    if args.dump_outputs:
+        x_last = x_dev.cpu().numpy() if world == 1 else torch.stack(out).cpu().numpy()
     ms_step = ms_total / args.steps / nirs  # per APPLY (a refinement step holds nirs of them)
 
     # ---- FGMRES-HIFIR solve time on every rank (second half of BASELINE.json's metric)
@@ -658,7 +702,7 @@ def run_ours(args, rank, world, local_rank):
             t0 = time.perf_counter()
             _, rflag, riters, rnmv = M.krylov(bk, "fgmres")
             extra["fgmres"].update(cpu_time_s=time.perf_counter() - t0, cpu_iters=riters, cpu_num_mv=rnmv,
-                                   cpu_threads=threads)
+                                   cpu_threads=1)
 
     # ---- the other BASELINE configs (3, 4, 5) as sub-records, measured on every rank
     st = G.stats()
@@ -671,11 +715,10 @@ def run_ours(args, rank, world, local_rank):
     cpu = None
     if rank == 0 and world == 1 and not args.no_cpu:
         applies = max(1, args.cpu_applies // nirs)
-        rate, dt = cpu_apply_rate(M, n, applies, nirs=nirs, A=A)
-        cpu = {"value": rate * nirs, "unit": "applies/s", "cores": 1 if nirs <= 1 else threads, "kind": "reference",
-               "sample": (f"{applies} hif::HIF::solve applies" if nirs <= 1 else
-                          f"{applies} hif::HIF::hifir(nirs={nirs}) solves (A x with {threads} OpenMP threads)") +
-                         f" of the same workload on the same factorized object ({dt:.1f} s; the reference apply is serial)"}
+        rate, dt, _ = cpu_apply_rate(M, n, applies, nirs=nirs, A=A)
+        cpu = {"value": rate * nirs, "unit": "applies/s", "cores": 1, "kind": "oracle",
+               "sample": (f"{applies} C oracle applies" if nirs <= 1 else f"{applies} C oracle hifir(nirs={nirs}) solves") +
+                         f" of the same workload on the same factors ({dt:.1f} s, serial)"}
     arena = None
     if args.arena_check and world == 1:
         # factor arena file (csrc/arena.cu): write, attach from the file, compare with the live attach
@@ -721,7 +764,7 @@ def run_ours(args, rank, world, local_rank):
             r0 = dict(allrec[0])
             ms = statistics.median([max(r["local_ms"][i] for r in allrec) for i in range(len(r0["local_ms"]))])  # max over ranks
             r0.pop("local_ms")
-            r0["parity_vs_reference"] = max(r["parity_vs_reference"] for r in allrec)
+            r0["parity_vs_oracle"] = max(r["parity_vs_oracle"] for r in allrec)
             r0["ms_per_step"] = ms / r0["steps"]
             peak = hbm_peak()[0]
             if kind == "mrhs":
@@ -796,7 +839,7 @@ def run_ours(args, rank, world, local_rank):
         "data": "synthetic",
         "config": {"workload": workload_name(args.workload, args.size, 1) + (" single-precision factors" if single else "")
                    + (f" hifir nirs={nirs}" if nirs > 1 else ""),
-                   "n": n, "params": "tau=1e-2 alpha=3 kappa=5 (reference PDE set)", "l2_policy": L2_POLICY},
+                   "n": n, "params": FACTORS, "l2_policy": L2_POLICY},
         "run": {"levels": st["levels"], "nnz_factors": st["nnz"],
                 "l2_policy": f"inputs larger than L2: {bytes_apply / 1e9:.2f} GB streamed per apply vs 126 MB L2",
                 "parallelism": "replicas, independent right-hand sides per GPU" if world > 1 else "1 GPU",
@@ -809,7 +852,7 @@ def run_ours(args, rank, world, local_rank):
                         "steps overlap; every step copies its b in and its x out)") if pipelined else
                        ((("lhfsdGpuSolve" if single else "lhfdGpuSolve") if nirs <= 1 else
                          ("lhfsdGpuApply" if single else "lhfdGpuApply") + f"(LHF_S, nirs={nirs})") + " (pinned host buffers)")},
-        "gpu_launches": launches, "clocks": clocks, "parity_vs_reference": parity,
+        "gpu_launches": launches, "clocks": clocks, "parity_vs_oracle": parity,
     }
     if arena:
         line["arena"] = arena
@@ -820,6 +863,8 @@ def run_ours(args, rank, world, local_rank):
                                  "independent systems per GPU"}
     line.update(extra)
     line.update(extras)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, x=x_last)
     print(json.dumps(line), flush=True)
 
 
@@ -840,7 +885,6 @@ def main():
     ap.add_argument("--arena-check", action="store_true",
                     help="also write a factor arena file, attach from it and compare (csrc/arena.cu)")
     ap.add_argument("--cpu-applies", type=int, default=40)
-    ap.add_argument("--ref-max-steps", type=int, default=300)
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-fgmres", action="store_true")
     ap.add_argument("--extras", default="mrhs,hifir,stokes",
@@ -848,8 +892,12 @@ def main():
                          "stokes (config 3); '' = none")
     ap.add_argument("--extra-steps", type=int, default=10)
     ap.add_argument("--extras-small", action="store_true", help="developer: small sizes for the extras")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float64, at most 64 MB in all)")
     args = ap.parse_args()
     args.warmup = max(3, args.warmup)
+    if args.dump_outputs and args.impl == "reference" and args.nrhs > 1:
+        ap.error("--dump-outputs: the batched reference arm applies in worker processes and returns no outputs")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -251,7 +251,7 @@ def test_level_merging_shortens_the_dependency_chain(lib, monkeypatch):
 REF_SRC = "/root/reference/src"
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF_SRC, "hifir.hpp")), reason="reference headers not on this box")
+@pytest.mark.skipif(not os.path.exists(os.path.join(REF_SRC, "hifir.hpp")), reason="needs the reference HIFIR headers, which this repository does not contain")
 def test_cxx_adapter_compiles_against_the_reference_headers(tmp_path):
     """include/hifir_b200.hpp next to the reference's own <hifir.hpp>: the link-time attach overloads for
     hif::HIF<double,int> and hif::HIF<float,int>, the entry-point-table form and describe() + SaveLevels

@@ -242,7 +242,7 @@ def test_linearity_and_zero_rhs():
 
 
 # ------------------------------------------------------------------ live reference
-needs_ref = pytest.mark.skipif(not have_reference(), reason="oracle/_ref/libhifir_ref.so not on this box")
+needs_ref = pytest.mark.skipif(not have_reference(), reason="needs oracle/_ref/libhifir_ref.so, built from the reference HIFIR sources, which this repository does not contain")
 
 
 def _attach_through_cxx_adapter(M):

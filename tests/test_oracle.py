@@ -124,7 +124,7 @@ def test_port_on_float_factors_matches_float_reference(golden_f32):
 
 
 # ---------------------------------------------------------------- live reference
-needs_ref = pytest.mark.skipif(not have_reference(), reason="oracle/_ref/libhifir_ref.so not built/loadable")
+needs_ref = pytest.mark.skipif(not have_reference(), reason="needs oracle/_ref/libhifir_ref.so, built from the reference HIFIR sources, which this repository does not contain")
 
 
 @needs_ref

@@ -19,7 +19,7 @@ def main():
     args = ap.parse_args()
     build.build()
     A = make_problem(args.workload, args.size)
-    M = factorize(A, threads=os.cpu_count() or 1)
+    M = factorize(A)
     G = hb.GpuHif(M.levels())
     print("sweep_bytes", G.stats()["sweep_bytes"], "sweep_entries", G.stats()["sweep_entries"])
     n = A[0]

@@ -72,7 +72,7 @@ def main():
         k, v = kv.split("=")
         os.environ[k] = v
     A = make_problem(args.workload, args.size)
-    M = factorize(A, threads=os.cpu_count() or 1)
+    M = factorize(A)
     G = hb.GpuHif(M.levels())
     n = A[0]
     b = torch.from_numpy(P.seeded_rhs(n, 0)).cuda()

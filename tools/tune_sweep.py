@@ -30,7 +30,7 @@ def main():
     args = ap.parse_args()
     build.build()
     A = make_problem(args.workload, args.size)
-    M = factorize(A, threads=os.cpu_count() or 1)
+    M = factorize(A)
     levels = M.levels()
     n = A[0]
     bh = P.seeded_rhs(n, 0)
