@@ -127,6 +127,7 @@ def lib():
             "lhfdGpuProfileSolveDev": [vp, vp, vp, sz, sz, vp, vp, vp, sz],
             "lhfdGpuDebugSweepHost": [vp, i, vp, vp, vp, vp],
             "lhfdGpuDebugPlanLab": [vp, i, vp, vp, vp],
+            "lhfdGpuDebugMergePlan": [vp, i, vp],
             "lhfdGpuDebugExportInts": [vp, sz, i, vp, sz, vp],
             "lhfdGpuDebugTraceSweep": [vp, vp, vp, i, i, vp, sz, vp],
             "lhfdGpuDebugSegmentGraph": [vp, i, sz, sz, vp, vp, vp],
@@ -172,6 +173,7 @@ EXPORTED_SYMBOLS = (
     "lhfdGpuSaveLevels", "lhfsGpuSaveLevels", "lhfdGpuAttachFile", "lhfsGpuAttachFile", "lhfGpuFileInfo")
 # developer / test hooks declared in hifir_b200/csrc/debug_api.h (not part of the drop-in boundary)
 DEBUG_SYMBOLS = ("lhfdGpuDebugSweepHost", "lhfsGpuDebugSweepHost", "lhfGpuDebugFileSweepHost", "lhfdGpuDebugPlanLab",
+                 "lhfdGpuDebugMergePlan",
                  "lhfdGpuDebugExportInts", "lhfdGpuDebugTraceSweep", "lhfdGpuDebugSegmentGraph",
                  "lhfdGpuDebugNorm2Dev")
 
@@ -204,6 +206,22 @@ def debug_sweep_host(block, upper, rhs, diag=None):
     _chk(f(C.byref(c), int(upper), _ptr(rhs), _ptr(d) if d is not None else None,
                                      _ptr(x), _ptr(st)))
     return x, dict(zip(("slices", "padded", "bytes", "depth"), (int(v) for v in st)))
+
+
+MERGE_PLAN_KEYS = ("rows", "entries", "depth", "merged_rows", "merged_entries", "steps", "super_levels", "predicted_us")
+
+
+def debug_merge_plan(block, upper):
+    """Host-only hook (lhfdGpuDebugMergePlan): the attach-time merge plan of the triangular CCS block
+    under the current settings, with its predicted sweep time under the library's cost model."""
+    nr, nc, cs, ri, va = block
+    cs = np.ascontiguousarray(cs, dtype=np.int64)
+    ri = np.ascontiguousarray(ri, dtype=np.int32)
+    va = np.ascontiguousarray(va, dtype=np.float64)
+    c = LhfdGpuCcs(nr, nc, _ptr(cs), _ptr(ri), _ptr(va))
+    out = np.zeros(8)
+    _chk(lib().lhfdGpuDebugMergePlan(C.byref(c), int(upper), _ptr(out)))
+    return {k: (float(v) if k == "predicted_us" else int(v)) for k, v in zip(MERGE_PLAN_KEYS, out)}
 
 
 def debug_segment_graph(block, upper, max_segs=1 << 19, max_deps=1 << 26):

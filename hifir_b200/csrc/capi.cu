@@ -601,6 +601,34 @@ LhfStatus lhfdGpuDebugSweepHost(const LhfdGpuCcs *T, int upper, const double *rh
   });
 }
 
+LhfStatus lhfdGpuDebugMergePlan(const LhfdGpuCcs *T, int upper, double out[8]) {
+  REQUIRE_PTR(T, "T");
+  REQUIRE_PTR(out, "out");
+  return guarded([&] {
+    HostCsr R = ccs_to_csr(*T, "T");
+    R.nrows = R.ncols = T->ncols;
+    R.ptr.resize(T->ncols + 1, R.ptr.empty() ? 0u : R.ptr.back());
+    const MergeParams mp = MergeParams::from_env();
+    MergeStats        ms;
+    const HostCsr     S = merged_sweep_form(R, upper != 0, mp, &ms);
+    if (!mp.enabled) {  // the sweep form itself: one step per level set
+      std::vector<unsigned> lev(S.nrows, 0u);
+      std::size_t           depth = 0;
+      for (std::size_t i = 0; i < S.nrows; ++i) {
+        unsigned l = 0;
+        for (unsigned k = S.ptr[i]; k < S.ptr[i + 1]; ++k) l = std::max(l, lev[S.col[k]] + 1u);
+        lev[i] = l;
+        depth  = std::max<std::size_t>(depth, l + 1u);
+      }
+      ms.rows = ms.ext_rows = S.nrows, ms.nnz = ms.ext_nnz = S.col.size();
+      ms.depth = ms.ext_depth = ms.super_levels = depth;
+    }
+    const double v[8] = {double(ms.rows),      double(ms.nnz),          double(ms.depth),     double(ms.ext_rows),
+                         double(ms.ext_nnz),   double(ms.ext_depth),    double(ms.super_levels), mp.plan_cost(ms)};
+    std::copy(v, v + 8, out);
+  });
+}
+
 LhfStatus lhfdGpuDebugPlanLab(const LhfdGpuCcs *T, int upper, const int *key, const double *opts, double *out) {
   REQUIRE_PTR(T, "T");
   REQUIRE_PTR(opts, "opts");

@@ -29,6 +29,11 @@ LhfStatus lhfsGpuDebugSweepHost(const LhfsGpuCcs *T, int upper, const double *rh
 LhfStatus lhfGpuDebugFileSweepHost(const char *path, size_t level, int upper, const double *rhs, double *x,
                                    size_t stats[4]);
 
+/* Host only: the attach-time merge plan of the strictly triangular CCS block T (merge.cu) under the
+ * current settings.  out = {rows, entries, depth, merged rows, merged entries, merged depth (dependent
+ * steps), super levels, predicted time of one sweep in us under the committed cost model}. */
+LhfStatus lhfdGpuDebugMergePlan(const LhfdGpuCcs *T, int upper, double out[8]);
+
 /* Host only: gather-locality statistics of candidate row orders / slot numberings (planlab.cu). */
 LhfStatus lhfdGpuDebugPlanLab(const LhfdGpuCcs *T, int upper, const int *key, const double *opts, double *out);
 

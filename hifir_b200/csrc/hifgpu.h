@@ -93,8 +93,22 @@ struct MergeParams {
   bool     slack     = false;     // slack-aware merging (merge_slack): only rows pinned to the critical core pay fill
   unsigned steps     = 0;         // > 0: proportional scheduling into this many steps (merge_prop)
   bool     chain_all = true;      // chain every row (not only the pinned ones) to the t rows of the previous step
-  bool     auto_caps = true;      // choose sl_cap / gain from the size of the factor (merge_levels)
+  bool     auto_caps = true;      // choose sl_cap per factor with the cost model below (merge_levels)
+  // Cost model of one warp-stream sweep over a plan (us, B200 at 1000 W):
+  //   t = tau_step * dependent steps + c_entry * stored entries
+  // [0]: the packed plan (~12 B per entry + 8 B per row) is larger than l2_bytes and streams from HBM,
+  // [1]: it stays L2-resident.  Least-squares fit to the merge-cap curve of Poisson 128^3 (fused L-then-U
+  // launches of all four levels, 9 plans each; profiles/r03_tune_poisson128.log): rms error 21 us over
+  // 13 launches of 370-1000 us [0], 30 us over 23 launches of 47-1200 us [1].  A small factor does not
+  // fill the machine, so its entries cost six times more: fill pays off far earlier than in a large one.
+  double   tau_step[2] = {1.31, 1.11};
+  double   c_entry[2]  = {3.44e-6, 2.13e-5};
+  double   l2_bytes    = 40.0e6;
   static MergeParams from_env();
+  // predicted time of one sweep over a plan with these statistics
+  double plan_cost(std::size_t steps, std::size_t entries, std::size_t rows) const;
+  template <class St>
+  double plan_cost(const St &s) const { return plan_cost(s.ext_depth, s.ext_nnz, s.ext_rows); }
 };
 struct MergeStats {
   std::size_t rows = 0, ext_rows = 0, nnz = 0, ext_nnz = 0, depth = 0, ext_depth = 0, super_levels = 0;

@@ -47,6 +47,12 @@ MergeParams MergeParams::from_env() {
   return p;
 }
 
+double MergeParams::plan_cost(std::size_t steps, std::size_t entries, std::size_t rows) const {
+  const double e = static_cast<double>(entries), r = static_cast<double>(rows);
+  const int    k = 12.0 * e + 8.0 * r <= l2_bytes ? 1 : 0;
+  return tau_step[k] * static_cast<double>(steps) + c_entry[k] * e;
+}
+
 // Rows in sweep order (forward for L, backward for U), every entry references an EARLIER row,
 // entries of a row in the order the reference's column sweep applies them.
 HostCsr to_sweep_form(const HostCsr &T, bool upper) {
@@ -508,16 +514,49 @@ HostCsr merge_prop(const HostCsr &S, const MergeParams &prm, MergeStats *st) {
 HostCsr merge_levels(const HostCsr &S, const MergeParams &prm, MergeStats *st, bool fan_out) {
   const unsigned m = static_cast<unsigned>(S.nrows);
   if (S.gid.size() != m || S.orig_rows != m) throw std::logic_error("merge_levels: input is not in sweep form");
-  if (prm.auto_caps) {
-    // Per-factor caps (measured at Poisson 128^3 on the warp-stream sweep): a large factor keeps the
-    // machine busy between two dependent steps, so it pays for fewer, fatter steps (L_0 / U_0, 14 M
-    // entries: sl_cap 1e6 -> 133 / 156 us per sweep instead of 157 / 162); a small one is bound by the
-    // hops and more fill only costs (L_1 / U_1, 4 M entries: 3e5 -> 67 / 84 us instead of 76 / 84).
-    MergeParams q = prm;
-    q.auto_caps   = false;
-    q.sl_cap      = std::min(1.2e6, std::max(3.0e5, static_cast<double>(S.col.size()) / 14.0));
-    q.gain        = std::max(prm.gain, 3.0 * q.sl_cap);
-    return merge_levels(S, q, st, fan_out);
+  if (prm.auto_caps && prm.enabled && !prm.steps && !prm.slack) {
+    // Per-factor caps chosen by the cost model (MergeParams::plan_cost).  A super level that grows by
+    // k level sets fills every row with its dependency cone inside the super level (~k^3 entries for
+    // a stencil wavefront), so how much fill a saved step is worth depends on how the factor's
+    // entries and steps price on the device.  The candidates are tried from the most fill down:
+    // first the former fixed rule, sl_cap = clamp(nnz / 14, 3e5, 1.2e6) with gain = 3 sl_cap (fitted
+    // on factors with 3x more entries), then smaller caps, then the unmerged factor.  The first one
+    // that predicts a longer sweep than its predecessor ends the search (the curve has one minimum)
+    // and the cheapest plan seen is kept: deterministic, and a large factor -- whose minimum is near
+    // the top -- pays for two or three plans at attach, the cheaper ones to build.
+    const double kCaps[] = {std::min(1.2e6, std::max(3.0e5, static_cast<double>(S.col.size()) / 14.0)), 1e5, 3e4,
+                            1e4, 3e3, 1e3};
+    double       best = 0.0, prev = 0.0;
+    HostCsr      E;
+    MergeStats   est;
+    bool         turned = false;
+    for (double cap : kCaps) {
+      MergeParams q = prm;
+      q.auto_caps   = false;
+      q.sl_cap      = cap;
+      q.gain        = std::max(prm.gain, 3.0 * cap);  // the super level's size binds, not one level set's fill
+      MergeStats    qs;
+      HostCsr       Q = merge_levels(S, q, &qs, fan_out);
+      const double  c = prm.plan_cost(qs);
+      if (cap == kCaps[0] || c < best) best = c, E = std::move(Q), est = qs;
+      if (cap != kCaps[0] && c > prev) {
+        turned = true;
+        break;
+      }
+      prev = c;
+    }
+    if (!turned) {  // still falling: the unmerged factor
+      std::vector<unsigned> lev;
+      const std::size_t     depth0 = depth_of(S, lev);
+      if (prm.plan_cost(depth0, S.col.size(), m) < best) {
+        E        = S;
+        est.rows = est.ext_rows = m;
+        est.nnz = est.ext_nnz = S.col.size();
+        est.depth = est.ext_depth = est.super_levels = depth0;
+      }
+    }
+    if (st) *st = est;
+    return E;
   }
   if (prm.steps) return merge_prop(S, prm, st);
   if (prm.slack) return merge_slack(S, prm, st);

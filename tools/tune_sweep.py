@@ -75,7 +75,7 @@ def main():
             st = G.stats()
             print(f"[{cfg}] apply {ms:.3f} ms  parity {err:.1e}  attach {t_attach:.1f}s  device {st['device_bytes'] / 1e9:.2f} GB",
                   flush=True)
-            print("    " + " ".join(f"{k}={v * 1e3:.0f}" for k, v in prof.items() if v * 1e3 >= 8), flush=True)
+            print("    " + " ".join(f"{k}={v * 1e3:.1f}" for k, v in prof.items() if v * 1e3 >= 1), flush=True)
         except Exception as e:  # noqa: BLE001
             print(f"[{cfg}] failed: {e}", flush=True)
         G.close() if hasattr(G, "close") else None
