@@ -119,10 +119,13 @@ def lib():
             "lhfdGpuSolveMrhs": [vp, sz, vp, vp],
             "lhfdGpuFgmres": [vp, vp, i, d, i, i, vp, vp, vp, vp],
             "lhfdGpuGmres": [vp, vp, i, d, i, vp, vp, vp],
+            "lhfdGpuFgmresMrhs": [vp, sz, vp, i, d, i, i, vp, vp, vp, vp],
+            "lhfdGpuGmresMrhs": [vp, sz, vp, i, d, i, vp, vp, vp],
             "lhfdGpuApplyDev": [vp, i, vp, i, i, vp],
             "lhfdGpuSolveDev": [vp, vp, vp, sz],
             "lhfdGpuSolveMrhsDev": [vp, sz, vp, vp, sz],
             "lhfdGpuHifirDev": [vp, vp, sz, vp, sz],
+            "lhfdGpuHifirMrhsDev": [vp, sz, vp, sz, vp, sz],
             "lhfdGpuSpmvDev": [vp, vp, vp],
             "lhfdGpuProfileSolveDev": [vp, vp, vp, sz, sz, vp, vp, vp, sz],
             "lhfdGpuDebugSweepHost": [vp, i, vp, vp, vp, vp],
@@ -165,7 +168,8 @@ def lib():
 EXPORTED_SYMBOLS = (
     "lhfdGpuAttachLevels", "lhfdGpuDestroy", "lhfdGpuSetMatrix", "lhfdGpuSetNspConst", "lhfdGpuSetNspTranConst", "lhfdGpuClearNsp",
     "lhfdGpuSetStream", "lhfdGpuSynchronize", "lhfdGpuSolve", "lhfdGpuSolveAsync", "lhfdGpuApply", "lhfdGpuSolveMrhs",
-    "lhfdGpuFgmres", "lhfdGpuGmres", "lhfdGpuApplyDev", "lhfdGpuSolveDev", "lhfdGpuSolveMrhsDev", "lhfdGpuHifirDev",
+    "lhfdGpuFgmres", "lhfdGpuGmres", "lhfdGpuFgmresMrhs", "lhfdGpuGmresMrhs",
+    "lhfdGpuApplyDev", "lhfdGpuSolveDev", "lhfdGpuSolveMrhsDev", "lhfdGpuHifirDev", "lhfdGpuHifirMrhsDev",
     "lhfdGpuSpmvDev", "lhfdGpuProfileSolveDev",
     "lhfdGpuGetStats", "lhfdGpuGetDepths", "lhfGpuGetErrorMsg", "lhfGpuVersion",
     "lhfsGpuAttachLevels", "lhfsGpuDestroy", "lhfsGpuAsDouble", "lhfsGpuSetMatrix", "lhfsdGpuUpdate", "lhfsGpuSolve",
@@ -433,6 +437,29 @@ class GpuHif:
                                 C.byref(iters)))
         return x, flag.value, iters.value
 
+    def _block(self, B):
+        B = np.ascontiguousarray(B, dtype=np.float64)
+        assert B.ndim == 2 and B.shape[0] == self.n
+        k = B.shape[1]
+        return B, np.empty_like(B), np.zeros(k, dtype=np.int32), np.zeros(k, dtype=np.int32), np.zeros(k, dtype=np.int32)
+
+    def fgmres_mrhs(self, B, restart=30, rtol=1e-6, maxit=500, full_rank=False):
+        """lhfdGpuFgmresMrhs: one fgmres per column of the (n, nrhs) block B, run together on the batched
+        apply.  Returns (X, flags, iters, num_mv), the last three arrays of nrhs entries."""
+        B, X, flags, iters, nmv = self._block(B)
+        if B.shape[1]:
+            _chk(lib().lhfdGpuFgmresMrhs(self._h, B.shape[1], _ptr(B), restart, rtol, maxit, int(full_rank), _ptr(X),
+                                         _ptr(flags), _ptr(iters), _ptr(nmv)))
+        return X, flags, iters, nmv
+
+    def gmres_mrhs(self, B, restart=30, rtol=1e-6, maxit=500):
+        """lhfdGpuGmresMrhs: one gmres per column of the (n, nrhs) block B.  Returns (X, flags, iters)."""
+        B, X, flags, iters, _ = self._block(B)
+        if B.shape[1]:
+            _chk(lib().lhfdGpuGmresMrhs(self._h, B.shape[1], _ptr(B), restart, rtol, maxit, _ptr(X), _ptr(flags),
+                                        _ptr(iters)))
+        return X, flags, iters
+
     # ---- device-pointer entry points (ints = raw device addresses, e.g. tensor.data_ptr()) ----
     def solve_dev(self, d_b, d_x, rank=0):
         _chk(lib().lhfdGpuSolveDev(self._h, C.c_void_p(d_b), C.c_void_p(d_x), rank))
@@ -445,6 +472,10 @@ class GpuHif:
 
     def hifir_dev(self, d_b, nirs, d_x, rank=FULL_RANK):
         _chk(lib().lhfdGpuHifirDev(self._h, C.c_void_p(d_b), nirs, C.c_void_p(d_x), rank))
+
+    def hifir_mrhs_dev(self, nrhs, d_B, nirs, d_X, rank=FULL_RANK):
+        """lhfdGpuHifirMrhsDev: hifir_dev on a row-interleaved (n, nrhs) device block"""
+        _chk(lib().lhfdGpuHifirMrhsDev(self._h, nrhs, C.c_void_p(d_B), nirs, C.c_void_p(d_X), rank))
 
     def profile_solve_dev(self, d_b, d_x, rank=0):
         """Instrumented apply: [(label, milliseconds)] for every kernel of the schedule."""

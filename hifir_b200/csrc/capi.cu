@@ -547,6 +547,54 @@ LhfStatus lhfdGpuGmres(LhfdGpuHdl hdl, const double *b, int restart, double rtol
   return krylov_host(hdl, false, b, restart, rtol, maxit, 0, x, flag, iters, nullptr);
 }
 
+// nrhs independent Krylov solves on one row-interleaved host block (krylov_mrhs_dev); nrhs == 1 is krylov_host
+static LhfStatus krylov_mrhs_host(LhfdGpuHdl hdl, bool flexible, size_t nrhs, const double *B, int restart, double rtol,
+                                  int maxit, int full_rank, double *X, int *flag, int *iters, int *num_mv) {
+  REQUIRE_HANDLE(hdl);
+  REQUIRE_PTR(B, "B");
+  REQUIRE_PTR(X, "X");
+  if (!nrhs) return LHF_SUCCESS;
+  return guarded([&] {
+    Handle *h = H(hdl);
+    if (h->nsp_on) throw std::logic_error("multiple RHS does not support null space filter.");  // builder.hpp:440
+    HIF_CUDA(cudaSetDevice(h->device));
+    check_krylov_mrhs(h, nrhs, restart);  // before the staging buffers are sized for the block
+    ensure_io(h, nrhs);
+    h2d(h, h->io_b.p, B, h->n0() * nrhs);
+    std::vector<int> f(nrhs), it(nrhs), nmv(nrhs);
+    krylov_mrhs_dev(h, flexible, nrhs, h->io_b.p, restart, rtol, maxit, full_rank != 0, h->io_x.p, f.data(), it.data(),
+                    nmv.data());
+    d2h(h, X, h->io_x.p, h->n0() * nrhs);
+    check_sweep_error(h);
+    if (flag) std::copy(f.begin(), f.end(), flag);
+    if (iters) std::copy(it.begin(), it.end(), iters);
+    if (num_mv) std::copy(nmv.begin(), nmv.end(), num_mv);
+  });
+}
+
+LhfStatus lhfdGpuFgmresMrhs(LhfdGpuHdl hdl, size_t nrhs, const double *B, int restart, double rtol, int maxit,
+                            int full_rank, double *X, int *flag, int *iters, int *num_mv) {
+  return krylov_mrhs_host(hdl, true, nrhs, B, restart, rtol, maxit, full_rank, X, flag, iters, num_mv);
+}
+
+LhfStatus lhfdGpuGmresMrhs(LhfdGpuHdl hdl, size_t nrhs, const double *B, int restart, double rtol, int maxit,
+                           double *X, int *flag, int *iters) {
+  return krylov_mrhs_host(hdl, false, nrhs, B, restart, rtol, maxit, 0, X, flag, iters, nullptr);
+}
+
+LhfStatus lhfdGpuHifirMrhsDev(LhfdGpuHdl hdl, size_t nrhs, const double *d_B, size_t nirs, double *d_X, size_t rank) {
+  REQUIRE_HANDLE(hdl);
+  REQUIRE_PTR(d_B, "B");
+  REQUIRE_PTR(d_X, "X");
+  if (!nrhs) return LHF_SUCCESS;
+  return guarded([&] {
+    Handle *h = H(hdl);
+    if (h->nsp_on) throw std::logic_error("multiple RHS does not support null space filter.");  // builder.hpp:440
+    HIF_CUDA(cudaSetDevice(h->device));
+    hifir_mrhs_dev(h, nrhs, d_B, nirs, d_X, rank);
+  });
+}
+
 LhfStatus lhfdGpuProfileSolveDev(LhfdGpuHdl hdl, const double *d_b, double *d_x, size_t rank, size_t max_entries,
                                  float *ms, size_t *count, char *names, size_t names_len) {
   REQUIRE_HANDLE(hdl);

@@ -303,6 +303,11 @@ struct Handle {
   DevBuf<unsigned long long> kr_bar;
   unsigned long long         kr_bar_base = 0;
   bool                       kr_no_coop  = false;  // the cooperative launch was refused once: per-step kernels from then on
+  // block Krylov (krylov.cu): bases [restart][n][nrhs] (Z: FGMRES only), [n][nrhs] work blocks, per-column
+  // scalars (Hessenberg column [restart+1][nrhs], y [restart][nrhs], norms), block partials, retired-column mask
+  DevBuf<double>   kb_Q, kb_Z, kb_v, kb_w, kb_r, kb_t, kb_H, kb_y, kb_red, kb_part;
+  DevBuf<int>      kb_mask;
+  DevBuf<unsigned> kb_count;  // arrival counter of mgs_step_cols_kernel
   double *       h_scal = nullptr;  // pinned
   int            kr_restart = 0;
   // multi-rhs column staging
@@ -372,6 +377,11 @@ void   hifir_betas_dev(Handle *h, const double *d_b, std::size_t nirs, const dou
 void   krylov_dev(Handle *h, bool flexible, const double *d_b, int restart, double rtol, int maxit,
                   bool full_rank, double *d_x, int *flag, int *iters, int *num_mv);
 double norm2_dev(Handle *h, const double *d_v, std::size_t n);
+// the same on row-interleaved blocks of nrhs columns (nrhs == 1: the single-rhs functions above)
+void   check_krylov_mrhs(Handle *h, std::size_t nrhs, int restart);  // matrix, restart and block size
+void   hifir_mrhs_dev(Handle *h, std::size_t nrhs, const double *d_B, std::size_t nirs, double *d_X, std::size_t rank);
+void   krylov_mrhs_dev(Handle *h, bool flexible, std::size_t nrhs, const double *d_B, int restart, double rtol, int maxit,
+                       bool full_rank, double *d_X, int *flag, int *iters, int *num_mv);
 
 // ---- wsweep.cu : statically scheduled warp-stream sweeps
 struct WsHost {  // packed plan on the host

@@ -169,6 +169,16 @@ LhfStatus lhfdGpuFgmres(LhfdGpuHdl hdl, const double *b, int restart, double rto
 LhfStatus lhfdGpuGmres(LhfdGpuHdl hdl, const double *b, int restart, double rtol, int maxit,
                        double *x, int *flag, int *iters);
 
+/* nrhs independent fgmres_hifir / gmres_hif solves with one matrix and one preconditioner.
+ * B and X are row-interleaved, B[i*nrhs + k].  flag / iters / num_mv are arrays of nrhs
+ * entries, or NULL.  The per-column meaning is that of lhfdGpuFgmres / lhfdGpuGmres.
+ * The columns run in lockstep on the batched apply; nrhs == 1 is lhfdGpuFgmres / lhfdGpuGmres.
+ * nrhs == 0 is a no-op; a null-space filter is refused (as lhfdGpuSolveMrhs). */
+LhfStatus lhfdGpuFgmresMrhs(LhfdGpuHdl hdl, size_t nrhs, const double *B, int restart, double rtol,
+                            int maxit, int full_rank, double *X, int *flag, int *iters, int *num_mv);
+LhfStatus lhfdGpuGmresMrhs(LhfdGpuHdl hdl, size_t nrhs, const double *B, int restart, double rtol,
+                           int maxit, double *X, int *flag, int *iters);
+
 /* ---- single-precision factors: hif::HIF<float> (libhifir's lhfs* family, libhifir.h:775-872)
  * and the mixed-precision lhfsd* family (float factors, double vectors; libhifir.h:1231-1280,
  * libhifir.cpp:1192-1229, examples/intermediate/demo_mixedprecision.cpp) ------------------------
@@ -259,6 +269,9 @@ LhfStatus lhfdGpuSolveMrhsDev(LhfdGpuHdl hdl, size_t nrhs, const double *d_B, do
 /* hif::HIF::hifir fixed-count variant (builder.hpp:458-465, IterRefine.hpp:77-105) */
 LhfStatus lhfdGpuHifirDev(LhfdGpuHdl hdl, const double *d_b, size_t nirs, double *d_x,
                           size_t rank);
+/* hif::HIF::hifir, fixed count (as lhfdGpuHifirDev), on a row-interleaved device block */
+LhfStatus lhfdGpuHifirMrhsDev(LhfdGpuHdl hdl, size_t nrhs, const double *d_B, size_t nirs,
+                              double *d_X, size_t rank);
 /* y = A x with the matrix given to lhfdGpuSetMatrix (mt::multiply_nt, mt_mv.hpp:57-73) */
 LhfStatus lhfdGpuSpmvDev(LhfdGpuHdl hdl, const double *d_x, double *d_y);
 
