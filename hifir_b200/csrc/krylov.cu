@@ -567,8 +567,11 @@ void krylov_dev(Handle *h, bool flexible, const double *d_b, int restart, double
 // (the layout of apply_mrhs_dev).  Every kernel below handles all columns in one launch.  Thread mapping: a
 // warp covers cw consecutive columns (cw = the smallest power of two >= nc, at most 32) of 32 / cw
 // consecutive rows, so every access of a row moves its cw values together; blockIdx.y selects a group of 32
-// columns when nc > 32.  A column's arithmetic and fold order depend on n and cw only -- never on the values
-// of the other columns or on the position the column holds.  mask[c] == 0 marks a retired column: the SpMV and
+// columns when nc > 32.  A column's arithmetic and fold order depend on n, cw and the number of column groups
+// ceil(nc / 32) only -- never on the values of the other columns or on the position the column holds.  The
+// groups enter through the row blocks of the reductions, nb_red = min(kRB / groups, ceil(n / rows_cta)) of
+// col_shape: at n = 262 144 and cw = 32 that is 592, 296 or 197 blocks for 1, 2 or 3 groups, so the same
+// column folds in another order in a block of another width.  mask[c] == 0 marks a retired column: the SpMV and
 // the reductions give 0 for it and the divisions write 0, so its basis vectors stay exact zeros.
 __device__ __forceinline__ void col_lane(unsigned cw, unsigned &c, unsigned &r0, unsigned &rstride) {
   const unsigned lane = threadIdx.x & 31u, rw = 32u / cw;
