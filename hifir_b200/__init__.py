@@ -128,7 +128,8 @@ def lib():
             "lhfdGpuHifirMrhsDev": [vp, sz, vp, sz, vp, sz],
             "lhfdGpuSpmvDev": [vp, vp, vp],
             "lhfdGpuProfileSolveDev": [vp, vp, vp, sz, sz, vp, vp, vp, sz],
-            "lhfdGpuDebugSweepHost": [vp, i, vp, vp, vp, vp],
+            "lhfdGpuDebugSweepHost": [vp, i, vp, vp, vp, vp, i],
+            "lhfdGpuDebugSweepDev": [vp, i, sz, i, vp, vp, vp, vp, sz, vp, vp, vp],
             "lhfdGpuDebugPlanLab": [vp, i, vp, vp, vp],
             "lhfdGpuDebugMergePlan": [vp, i, vp],
             "lhfdGpuDebugExportInts": [vp, sz, i, vp, sz, vp],
@@ -145,7 +146,7 @@ def lib():
             "lhfsGpuApply": [vp, i, vp, i, vp, i, vp, vp],
             "lhfsdGpuSolve": [vp, vp, vp],
             "lhfsdGpuApply": [vp, i, vp, i, vp, i, vp, vp],
-            "lhfsGpuDebugSweepHost": [vp, i, vp, vp, vp, vp],
+            "lhfsGpuDebugSweepHost": [vp, i, vp, vp, vp, vp, i],
             "lhfdGpuSaveLevels": [sz, vp, i, C.c_char_p],
             "lhfsGpuSaveLevels": [sz, vp, i, C.c_char_p],
             "lhfdGpuAttachFile": [i, C.c_char_p, vp],
@@ -179,7 +180,7 @@ EXPORTED_SYMBOLS = (
 DEBUG_SYMBOLS = ("lhfdGpuDebugSweepHost", "lhfsGpuDebugSweepHost", "lhfGpuDebugFileSweepHost", "lhfdGpuDebugPlanLab",
                  "lhfdGpuDebugMergePlan",
                  "lhfdGpuDebugExportInts", "lhfdGpuDebugTraceSweep", "lhfdGpuDebugSegmentGraph",
-                 "lhfdGpuDebugNorm2Dev")
+                 "lhfdGpuDebugNorm2Dev", "lhfdGpuDebugSweepDev")
 
 
 class LhfError(RuntimeError):
@@ -193,9 +194,10 @@ def _chk(st):
         raise LhfError(st, (lib().lhfGpuGetErrorMsg() or b"").decode())
 
 
-def debug_sweep_host(block, upper, rhs, diag=None):
+def debug_sweep_host(block, upper, rhs, diag=None, parity=None):
     """Host-only hook (lhfdGpuDebugSweepHost): merge and pack the triangular CCS block as attach
-    does and solve with the packed data on the CPU.  Returns (x, stats dict)."""
+    does and solve with the packed data on the CPU.  parity 0 / 1: every published value carries the
+    device's readiness tag.  Returns (x, stats dict)."""
     nr, nc, cs, ri, va = block
     single = np.asarray(va).dtype == np.float32  # float block -> lhfsGpuDebugSweepHost (values stored as float)
     cs = np.ascontiguousarray(cs, dtype=np.int64)
@@ -207,8 +209,8 @@ def debug_sweep_host(block, upper, rhs, diag=None):
     st = np.zeros(4, dtype=np.uint64)
     d = None if diag is None else np.ascontiguousarray(diag, dtype=np.float64)
     f = lib().lhfsGpuDebugSweepHost if single else lib().lhfdGpuDebugSweepHost
-    _chk(f(C.byref(c), int(upper), _ptr(rhs), _ptr(d) if d is not None else None,
-                                     _ptr(x), _ptr(st)))
+    _chk(f(C.byref(c), int(upper), _ptr(rhs), _ptr(d) if d is not None else None, _ptr(x), _ptr(st),
+           -1 if parity is None else int(parity)))
     return x, dict(zip(("slices", "padded", "bytes", "depth"), (int(v) for v in st)))
 
 
@@ -494,6 +496,27 @@ class GpuHif:
         _chk(lib().lhfdGpuDebugTraceSweep(self._h, C.c_void_p(d_b), C.c_void_p(d_x), level, which, _ptr(out),
                                           max_segs, C.byref(ns)))
         return out[: ns.value * 4].reshape(-1, 4)
+
+    SWEEP_FACTORS = ("L", "U", "LU")
+
+    def debug_sweep_dev(self, level, factor, rhs, transposed=False):
+        """lhfdGpuDebugSweepDev: one sweep of factor 'L', 'U' or 'LU' (the fused plan) of a level on the device,
+        next to the tag-exact host emulation of the plan the device holds.  rhs in original row order (m).
+        Returns dict(x, words, emul, slot_of, slot_of_l, parity): x (m) = the result rows as the apply reads
+        them, words / emul = the device's and the emulation's tagged words (uint64, slot order), slot_of = word
+        of every result row, slot_of_l = word of every row of the L part of a fused plan (else None)."""
+        rhs = np.ascontiguousarray(rhs, dtype=np.float64)
+        m = rhs.size
+        x = np.zeros(m)
+        words = np.zeros(4 * m, dtype=np.uint64)
+        emul = np.zeros(4 * m, dtype=np.uint64)
+        slot_of = np.zeros(2 * m, dtype=np.uint32)
+        nw, par = C.c_size_t(), C.c_uint()
+        _chk(lib().lhfdGpuDebugSweepDev(self._h, int(bool(transposed)), level, self.SWEEP_FACTORS.index(factor), _ptr(rhs),
+                                        _ptr(x), _ptr(words), _ptr(emul), words.size, C.byref(nw), _ptr(slot_of),
+                                        C.byref(par)))
+        return dict(x=x, words=words[: nw.value], emul=emul[: nw.value], slot_of=slot_of[:m],
+                    slot_of_l=slot_of[m:] if factor == "LU" else None, parity=par.value)
 
     def export_ints(self, level, which):
         """lhfdGpuDebugExportInts: a device-resident index array of one level, copied back

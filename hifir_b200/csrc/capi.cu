@@ -635,7 +635,7 @@ LhfStatus lhfdGpuProfileSolveDev(LhfdGpuHdl hdl, const double *d_b, double *d_x,
 }
 
 LhfStatus lhfdGpuDebugSweepHost(const LhfdGpuCcs *T, int upper, const double *rhs, const double *diag, double *x,
-                                size_t stats[4]) {
+                                size_t stats[4], int parity) {
   REQUIRE_PTR(T, "T");
   REQUIRE_PTR(rhs, "rhs");
   REQUIRE_PTR(x, "x");
@@ -645,7 +645,7 @@ LhfStatus lhfdGpuDebugSweepHost(const LhfdGpuCcs *T, int upper, const double *rh
     HostCsr R = ccs_to_csr(*T, "T");
     R.nrows = R.ncols = T->ncols;
     R.ptr.resize(T->ncols + 1, R.ptr.empty() ? 0u : R.ptr.back());
-    sweep_host_emulate(R, upper != 0, rhs, diag, x, stats);
+    sweep_host_emulate(R, upper != 0, rhs, diag, x, stats, false, parity < 0 ? -1 : parity & 1);
   });
 }
 
@@ -763,7 +763,7 @@ LhfStatus lhfGpuDebugFileSweepHost(const char *path, size_t level, int upper, co
 // single-precision factor block: widened, merged and packed as at attach, packed values rounded to
 // float (what the device streams), emulated on the host in double
 LhfStatus lhfsGpuDebugSweepHost(const LhfsGpuCcs *T, int upper, const double *rhs, const double *diag, double *x,
-                                size_t stats[4]) {
+                                size_t stats[4], int parity) {
   REQUIRE_PTR(T, "T");
   REQUIRE_PTR(rhs, "rhs");
   REQUIRE_PTR(x, "x");
@@ -776,7 +776,7 @@ LhfStatus lhfsGpuDebugSweepHost(const LhfsGpuCcs *T, int upper, const double *rh
     HostCsr             R = ccs_to_csr(Td, "T");
     R.nrows = R.ncols = T->ncols;
     R.ptr.resize(T->ncols + 1, R.ptr.empty() ? 0u : R.ptr.back());
-    sweep_host_emulate(R, upper != 0, rhs, diag, x, stats, true);
+    sweep_host_emulate(R, upper != 0, rhs, diag, x, stats, true, parity < 0 ? -1 : parity & 1);
   });
 }
 
@@ -826,6 +826,81 @@ LhfStatus lhfdGpuDebugTraceSweep(LhfdGpuHdl hdl, const double *d_b, double *d_x,
     const size_t ns = std::min<size_t>(plan.ws_nsegs, max_segs);
     HIF_CUDA(cudaMemcpy(out, h->trace_buf.p, ns * 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
     *nsegs = ns;
+  });
+}
+
+LhfStatus lhfdGpuDebugSweepDev(LhfdGpuHdl hdl, int transposed, size_t level, int which, const double *rhs, double *x,
+                               unsigned long long *words, unsigned long long *emul, size_t cap, size_t *nwords,
+                               unsigned *slot_of, unsigned *parity) {
+  REQUIRE_HANDLE(hdl);
+  REQUIRE_PTR(rhs, "rhs");
+  REQUIRE_PTR(x, "x");
+  REQUIRE_PTR(words, "words");
+  REQUIRE_PTR(emul, "emul");
+  REQUIRE_PTR(nwords, "nwords");
+  REQUIRE_PTR(slot_of, "slot_of");
+  REQUIRE_PTR(parity, "parity");
+  return guarded([&] {
+    Handle *h0 = H(hdl);
+    HIF_CUDA(cudaSetDevice(h0->device));
+    Handle *h = transposed ? handle_for_op(h0, LHF_SH) : h0;
+    if (level >= h->levels.size() || which < 0 || which > 2) throw std::invalid_argument("bad level / factor selector");
+    DevLevel &       D     = h->levels[level];
+    const bool       fused = which == 2;
+    const SweepPlan &plan  = fused ? D.LU : which == 1 ? D.U : D.L;
+    if (!plan.nblocks) throw std::invalid_argument("the handle launches no sweep of this factor (fused plans: which = 2)");
+    const std::size_t m = D.m, ns = 2 * m;  // every slot number is below 2 m (auxiliary unknowns: [m, 2 m))
+    if (cap < (fused ? 2 : 1) * ns) throw std::length_error("word buffers of 2 m entries (fused plan: 4 m) needed");
+    if (h->dbg_sweeps.size() < 3 * h->levels.size()) h->dbg_sweeps.resize(3 * h->levels.size());
+    Handle::DebugSweep &S = h->dbg_sweeps[3 * level + which];
+    if (!S.x1.p) {  // zeroed at allocation; the first call runs with parity 1, so the zeros never read as ready
+      S.x1.alloc(ns), S.x2.alloc(ns), S.rhs.alloc(ns), S.b.alloc(m), S.sync.alloc(h->tick_stride);
+      S.epoch = 0;
+    }
+    const unsigned par = ++S.epoch & 1u;
+    // what the sweep reads: b in original row order (L, fused), or the tagged input of a U sweep at the slots of
+    // the L plan (there the L sweep's result lives), divided by d permuted to the same slots
+    std::vector<double> rt(ns, tag_set_host(0.0, par)), dls(D.d_ls.n);
+    if (which == 1)
+      for (std::size_t r = 0; r < m; ++r) rt[D.L.slot_of.empty() ? r : D.L.slot_of[r]] = tag_set_host(rhs[r], par);
+    std::vector<double> xw((fused ? 2 : 1) * ns, 0.0), xe((fused ? 2 : 1) * ns, 0.0);
+    try {
+      HIF_CUDA(cudaMemcpyAsync(S.b.p, rhs, m * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+      HIF_CUDA(cudaMemcpyAsync(S.rhs.p, rt.data(), ns * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+      HIF_CUDA(cudaMemsetAsync(S.sync.p, 0, S.sync.n * sizeof(int), h->stream));
+      // the launch apply_schedule issues for this factor (launch_sweeps, apply.cu)
+      if (fused)
+        launch_ws_sweep(h, plan, S.b.p, nullptr, D.d_ls.p, S.x1.p, par, S.sync.p, nullptr, S.x2.p);
+      else if (which == 0)
+        launch_sweep(h, plan, S.b.p, nullptr, nullptr, S.x1.p, par, S.sync.p);
+      else
+        launch_sweep(h, plan, nullptr, S.rhs.p, D.d_ls.p, S.x1.p, par, S.sync.p);
+      check_sweep_error(h);
+      HIF_CUDA(cudaMemcpy(xw.data(), S.x1.p, ns * sizeof(double), cudaMemcpyDeviceToHost));
+      if (fused) HIF_CUDA(cudaMemcpy(xw.data() + ns, S.x2.p, ns * sizeof(double), cudaMemcpyDeviceToHost));
+    } catch (...) {
+      S = Handle::DebugSweep();  // slots left unwritten: start over with zeroed buffers on the next call
+      throw;
+    }
+    HIF_CUDA(cudaMemcpy(dls.data(), D.d_ls.p, dls.size() * sizeof(double), cudaMemcpyDeviceToHost));
+    const double *ein = which == 1 ? rt.data() : rhs;
+    if (plan.ws)
+      ws_emulate_device_plan(plan, ein, dls.data(), xe.data(), fused ? xe.data() + ns : nullptr, par);
+    else
+      stream_emulate_device_plan(plan, ein, dls.data(), xe.data(), par);
+    // words: the result buffer(s) in slot order, the fused plan's L buffer first; slot_of: word of every row
+    const std::size_t nl = fused ? D.L.ws_nslots : 0, nf = plan.ws ? (fused ? D.U.ws_nslots : plan.ws_nslots) : ns;
+    const std::vector<unsigned> &map = which == 0 ? D.L.slot_of : D.U.slot_of;
+    for (std::size_t k = 0; k < nl; ++k) std::memcpy(&words[k], &xw[k], 8), std::memcpy(&emul[k], &xe[k], 8);
+    for (std::size_t k = 0; k < nf; ++k)
+      std::memcpy(&words[nl + k], &xw[(fused ? ns : 0) + k], 8), std::memcpy(&emul[nl + k], &xe[(fused ? ns : 0) + k], 8);
+    for (std::size_t r = 0; r < m; ++r) {
+      slot_of[r] = static_cast<unsigned>(nl + (map.empty() ? r : map[r]));
+      if (fused) slot_of[m + r] = D.L.slot_of[r];
+      std::memcpy(&x[r], &words[slot_of[r]], 8);
+    }
+    *nwords = nl + nf;
+    *parity = par;
   });
 }
 

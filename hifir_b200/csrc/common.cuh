@@ -5,6 +5,7 @@
 
 #include <cstdint>
 #include <cstdio>
+#include <cstring>
 #include <stdexcept>
 #include <string>
 
@@ -42,6 +43,15 @@ __device__ __forceinline__ bool tag_ready(unsigned long long bits, unsigned pari
 }
 __device__ __forceinline__ double tag_value(unsigned long long bits) {
   return __longlong_as_double(static_cast<long long>(bits));
+}
+// host twin of tag_set for the emulations of the sweeps (wsweep.cu, stream.cu): the value a consumer
+// of the tagged word computes with
+inline double tag_set_host(double v, unsigned parity) {
+  unsigned long long b;
+  std::memcpy(&b, &v, 8);
+  b = (b & ~1ull) | parity;
+  std::memcpy(&v, &b, 8);
+  return v;
 }
 
 // polling load: must observe other SMs' stores -> L2 (never a stale L1 line)

@@ -13,16 +13,35 @@ extern "C" {
 #endif
 
 /* Host only: merges and packs the strictly triangular CCS block T exactly as attach does and solves
- * with the packed data on the CPU, segment by segment in the device's order: x = T^{-1} rhs (lower,
- * diag ignored) or x = T^{-1} (rhs ./ diag) (upper).  stats = {slices, padded entries, packed bytes,
- * dependency depth of the packed factor}. */
+ * with the packed data on the CPU, segment by segment in the device's arithmetic order: x = T^{-1} rhs
+ * (lower, diag ignored) or x = T^{-1} (rhs ./ diag) (upper).  stats = {slices, padded entries, packed
+ * bytes, dependency depth of the packed factor}.  parity < 0: plain values; 0 or 1: every published
+ * value (and the right-hand side of an upper sweep) carries the readiness tag of that parity in its
+ * last mantissa bit before it is read, as on the device. */
 LhfStatus lhfdGpuDebugSweepHost(const LhfdGpuCcs *T, int upper, const double *rhs, const double *diag,
-                                double *x, size_t stats[4]);
+                                double *x, size_t stats[4], int parity);
 
 /* The same for a single-precision factor block: the packed (merged) values are rounded to float
  * exactly as lhfsGpuAttachLevels stores them; rhs / diag / x are double. */
 LhfStatus lhfsGpuDebugSweepHost(const LhfsGpuCcs *T, int upper, const double *rhs, const double *diag,
-                                double *x, size_t stats[4]);
+                                double *x, size_t stats[4], int parity);
+
+/* One triangular sweep of an attached handle on the device, checked against the host emulation of the
+ * plan the device holds.  transposed != 0: the transposed twin (built on first use).  which: 0 = L,
+ * 1 = U, 2 = the fused L-then-U plan (attach fuses unless HIFIR_B200_WS_FUSE=0: then 0 and 1).  The
+ * launch is the one the apply issues for that factor, on the handle's stream, into tagged scratch
+ * buffers of the hook's own (per level and factor, zeroed at allocation, own epoch counter starting at
+ * parity 1): they hold the previous call's values under the other parity, as the apply's buffers do.
+ * rhs (m, original row order): b of L / fused, y of U (the sweep then solves U x = y ./ d; y enters
+ * tagged, as the L result does in the apply).  The packed plan is copied back from the device and
+ * emulated on the host, tag for tag, in an order its dataflow allows.
+ * Out: words / emul = the device's tagged result words and the emulation's, slot order (fused plan: the
+ * L buffer, then the U buffer), *nwords of them (cap >= 2 m, fused 4 m); slot_of[r] = word of row r of
+ * the result (fused plan: slot_of[m + r] = word of row r of the L part, slot_of has 2 m entries);
+ * x[r] = the result word of row r as the consumers of the apply read it (the tag bit included); parity. */
+LhfStatus lhfdGpuDebugSweepDev(LhfdGpuHdl hdl, int transposed, size_t level, int which, const double *rhs, double *x,
+                               unsigned long long *words, unsigned long long *emul, size_t cap, size_t *nwords,
+                               unsigned *slot_of, unsigned *parity);
 
 /* lhfdGpuDebugSweepHost on factor (level, upper) of an arena file, with the plan stored in the file
  * when it has one. */

@@ -318,6 +318,15 @@ struct Handle {
   // statistics
   std::size_t bytes_factors = 0, bytes_vec = 0, bytes_dense = 0, device_bytes = 0, nnz_total = 0;
   std::size_t kernels_per_apply = 0, launch_count = 0;
+  // debug: one triangular sweep on its own (lhfdGpuDebugSweepDev), per (level, factor) tagged scratch with its
+  // own epoch counter -- every tagged buffer is written exactly once per epoch, as the apply's are
+  struct DebugSweep {
+    DevBuf<unsigned long long> x1, x2, rhs;  // results (fused plan: L in x1, U in x2); tagged input of a U sweep
+    DevBuf<double>             b;            // plain right-hand side of an L / fused sweep
+    DevBuf<int>                sync;
+    unsigned                   epoch = 0;
+  };
+  std::vector<DebugSweep> dbg_sweeps;  // 3 per level: L, U, fused LU
   // debug: per-segment trace of one warp-stream sweep (lhfdGpuDebugTraceSweep)
   int                        trace_level = -1, trace_which = -1;
   DevBuf<unsigned long long> trace_buf;
@@ -343,14 +352,16 @@ HostCsr ccs_to_csr(const LhfdGpuCcs &c, const char *name);
 void build_sweep_plan(const HostCsr &T, bool upper, SweepPlan &plan, std::size_t *tally, unsigned nsm,
                       const unsigned *rhs_index = nullptr, int kind = -1);
 void sweep_host_emulate(const HostCsr &T, bool upper, const double *rhs, const double *diag, double *x,
-                        std::size_t stats[4], bool f32 = false);
+                        std::size_t stats[4], bool f32 = false, int parity = -1);
 void launch_sweep(Handle *h, const SweepPlan &plan, const double *rhs_plain, const unsigned long long *rhs_tagged,
                   const double *diag, unsigned long long *x, unsigned parity, int *sync,
                   unsigned nr = 0, unsigned long long *trace = nullptr);  // nr = 0: the plan's own width
 // ---- stream.cu
 void build_stream_plan(const HostCsr &S, bool upper, SweepPlan &plan, std::size_t *tally);
 void stream_host_emulate(const HostCsr &S, bool upper, const double *rhs, const double *diag, double *x,
-                         std::size_t stats[4], bool f32 = false);
+                         std::size_t stats[4], bool f32 = false, int parity = -1);
+// the emulation of a streaming plan on the arrays copied back from the device; x: 2 m entries
+void stream_emulate_device_plan(const SweepPlan &plan, const double *rhs, const double *diag, double *x, unsigned parity);
 void launch_stream_sweep(Handle *h, const SweepPlan &plan, const double *rhs_plain,
                          const unsigned long long *rhs_tagged, const double *diag, unsigned long long *x,
                          unsigned parity, int *ticket, unsigned long long *trace = nullptr, unsigned nr = 1);
@@ -386,20 +397,25 @@ void   krylov_mrhs_dev(Handle *h, bool flexible, std::size_t nrhs, const double 
 // ---- wsweep.cu : statically scheduled warp-stream sweeps
 struct WsHost {  // packed plan on the host
   unsigned                           nwarps = 0, nslots = 0, depth = 0, slices = 0;
-  std::vector<unsigned>              wdesc, stream, slot_of, order;  // order: (warp, absolute word offset) in creation order
+  std::vector<unsigned>              wdesc, stream, slot_of;
   std::vector<std::vector<unsigned>> seg_off;                        // per warp: word offsets of its segments (private stream)
   std::size_t                        entries = 0, padded = 0, copy_rows = 0, max_segs = 0, nsegs = 0;
 };
 void pack_warp_streams(const HostCsr &S, WsHost &H, unsigned nwarps, unsigned window, bool f32,
                        const unsigned *rhs_index, unsigned umin_force = 0);
 void ws_finalize_ring(WsHost &H, unsigned stages);
-void ws_host_emulate_packed(const WsHost &H, bool upper, bool f32, const double *rhs, const double *diag, double *x);
+// parity < 0: plain values; 0 / 1: published values carry the readiness tag as on the device (wsweep.cu)
+void ws_host_emulate_packed(const WsHost &H, bool upper, bool f32, const double *rhs, const double *diag, double *x,
+                            int parity = -1, double *x2 = nullptr);
+// the emulation of a warp-stream plan on the bytes copied back from the device (x2: U results of a fused plan)
+void ws_emulate_device_plan(const SweepPlan &plan, const double *rhs, const double *diag, double *x, double *x2,
+                            unsigned parity);
 void build_ws_plan(const HostCsr &S, bool upper, SweepPlan &plan, std::size_t *tally, unsigned nsm,
                    const unsigned *rhs_index, unsigned warps = 0, unsigned stages = 0);  // 0: HIFIR_B200_WS_WARPS / _STAGES
 void launch_ws_sweep_cols(Handle *h, const SweepPlan &plan, const double *rhs_plain, const double *diag, unsigned long long *xL,
                           unsigned long long *xU, unsigned parity, int *sync, unsigned nc);  // fused plan, nc = 16 | 32 | 64
 void ws_host_emulate(const HostCsr &S, bool upper, const double *rhs, const double *diag, double *x_by_row,
-                     std::size_t stats[4], bool f32);
+                     std::size_t stats[4], bool f32, int parity = -1);
 void launch_ws_sweep(Handle *h, const SweepPlan &plan, const double *rhs_plain, const unsigned long long *rhs_tagged,
                      const double *diag, unsigned long long *x, unsigned parity, int *sync,
                      unsigned long long *trace = nullptr, unsigned long long *x2 = nullptr);

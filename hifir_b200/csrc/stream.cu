@@ -449,43 +449,77 @@ void build_stream_plan(const HostCsr &S, bool upper, SweepPlan &plan, std::size_
   }
 }
 
-// CPU emulation of the streaming sweep on the packed data (slices in ticket order, rows of a
-// slice one after the other): lets tests check merge + packing without a GPU.  `x` has
-// 2 * orig_rows slots.  stats = {slices, padded entries, bytes, depth}
-void stream_host_emulate(const HostCsr &S, bool upper, const double *rhs, const double *diag, double *x,
-                         std::size_t stats[4], bool f32) {
-  StreamHost H;
-  pack_stream(S, H, stream_unroll());
-  if (f32)  // single-precision factors: the packed values are rounded to float (build_stream_plan)
-    for (double &v : H.vals) v = static_cast<double>(static_cast<float>(v));
-  const unsigned m = static_cast<unsigned>(S.orig_rows);
-  for (std::size_t s = 0; s < H.sdesc.size(); ++s) {
-    const uint4 sd = H.sdesc[s];
+namespace {
+// CPU emulation of the streaming sweep on packed arrays (slices in ticket order = level order, rows of a slice
+// one after the other), in the device's arithmetic order: per-lane fma over the entries, then the shfl_xor
+// tree.  `x` has 2 * m slots.  parity < 0: plain values; 0 / 1: every published value goes through tag_set
+// before any consumer reads it, and the right-hand side of an upper sweep (on the device the L sweep's
+// tagged result) is tagged as well.
+void stream_emulate_packed(const uint4 *sdesc, std::size_t nslices, const unsigned *codes, const unsigned *cols,
+                           const double *vals, unsigned m, bool upper, const double *rhs, const double *diag, double *x,
+                           int parity) {
+  auto pub = [&](double v) { return parity < 0 ? v : tag_set_host(v, static_cast<unsigned>(parity)); };
+  for (std::size_t s = 0; s < nslices; ++s) {
+    const uint4 sd = sdesc[s];
     if (sd.z == kEmptySlice) continue;
     const std::size_t base = static_cast<std::size_t>(sd.x) * 32u;
     const unsigned    lpr  = 1u << sd.z;
     for (unsigned lane = 0; lane < 32u; lane += lpr) {
-      const unsigned code = H.codes[s * 32u + lane];
+      const unsigned code = codes[s * 32u + lane];
       if (code == kPadCode) continue;
       const unsigned slot = code & kCodeSlotMask, ri = slot >= m ? slot - m : slot;
       double         part[32];
       for (unsigned j = 0; j < lpr; ++j) {  // per-lane partial sums, then the shuffle tree
-        double acc = (j == 0 && !(code & kCodeZeroRhs)) ? (upper ? rhs[ri] / diag[ri] : rhs[ri]) : 0.0;
+        double acc = (j == 0 && !(code & kCodeZeroRhs)) ? (upper ? pub(rhs[ri]) / diag[ri] : rhs[ri]) : 0.0;
         for (unsigned k = 0; k < sd.y; ++k) {
-          const unsigned c = H.cols[base + static_cast<std::size_t>(k) * 32u + lane + j];
-          if (c != kPadCol) acc = std::fma(-H.vals[base + static_cast<std::size_t>(k) * 32u + lane + j], x[c], acc);
+          const unsigned c = cols[base + static_cast<std::size_t>(k) * 32u + lane + j];
+          if (c != kPadCol) acc = std::fma(-vals[base + static_cast<std::size_t>(k) * 32u + lane + j], x[c], acc);
         }
         part[j] = acc;
       }
       for (unsigned o = lpr >> 1; o > 0; o >>= 1)
         for (unsigned j = 0; j < o; ++j) part[j] += part[j + o];
-      x[slot] = part[0];
+      x[slot] = pub(part[0]);
     }
   }
+}
+}  // namespace
+
+// CPU emulation of the streaming sweep on the packed data: lets tests check merge + packing without a GPU.
+// `x` has 2 * orig_rows slots.  stats = {slices, padded entries, bytes, depth}
+void stream_host_emulate(const HostCsr &S, bool upper, const double *rhs, const double *diag, double *x,
+                         std::size_t stats[4], bool f32, int parity) {
+  StreamHost H;
+  pack_stream(S, H, stream_unroll());
+  if (f32)  // single-precision factors: the packed values are rounded to float (build_stream_plan)
+    for (double &v : H.vals) v = static_cast<double>(static_cast<float>(v));
+  stream_emulate_packed(H.sdesc.data(), H.sdesc.size(), H.codes.data(), H.cols.data(), H.vals.data(),
+                        static_cast<unsigned>(S.orig_rows), upper, rhs, diag, x, parity);
   stats[0] = H.sdesc.size();
   stats[1] = H.padded;
   stats[2] = H.cols.size() * 12u + H.codes.size() * 4u + H.sdesc.size() * 16u;
   stats[3] = H.depth;
+}
+
+// the same on the arrays of a plan copied back from the device (float values widened, as the kernel does)
+void stream_emulate_device_plan(const SweepPlan &plan, const double *rhs, const double *diag, double *x, unsigned parity) {
+  if (!plan.nblocks) return;
+  std::vector<uint4>    sdesc(plan.st_sdesc.n / 4u);
+  std::vector<unsigned> codes(plan.st_codes.n), cols(plan.st_cols.n);
+  std::vector<double>   vals(plan.f32 ? plan.st_vals32.n : plan.st_vals.n);
+  if (codes.size() < sdesc.size() * 32u || vals.size() != cols.size()) throw std::logic_error("streaming plan: array sizes");
+  HIF_CUDA(cudaMemcpy(sdesc.data(), plan.st_sdesc.p, sdesc.size() * sizeof(uint4), cudaMemcpyDeviceToHost));
+  HIF_CUDA(cudaMemcpy(codes.data(), plan.st_codes.p, codes.size() * 4u, cudaMemcpyDeviceToHost));
+  HIF_CUDA(cudaMemcpy(cols.data(), plan.st_cols.p, cols.size() * 4u, cudaMemcpyDeviceToHost));
+  if (plan.f32) {
+    std::vector<float> v32(vals.size());
+    HIF_CUDA(cudaMemcpy(v32.data(), plan.st_vals32.p, v32.size() * 4u, cudaMemcpyDeviceToHost));
+    std::copy(v32.begin(), v32.end(), vals.begin());
+  } else {
+    HIF_CUDA(cudaMemcpy(vals.data(), plan.st_vals.p, vals.size() * 8u, cudaMemcpyDeviceToHost));
+  }
+  stream_emulate_packed(sdesc.data(), sdesc.size(), codes.data(), cols.data(), vals.data(), plan.m, plan.upper, rhs, diag, x,
+                        static_cast<int>(parity));
 }
 
 namespace {

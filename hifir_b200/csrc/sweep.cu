@@ -39,17 +39,17 @@ void build_sweep_plan(const HostCsr &Tnat, bool upper, SweepPlan &plan, std::siz
 // CPU emulation of a sweep on the packed data -- lets the host-side merging + packing be tested
 // without a GPU (tests/test_abi.py)
 void sweep_host_emulate(const HostCsr &T, bool upper, const double *rhs, const double *diag, double *x,
-                        std::size_t stats[4], bool f32) {
+                        std::size_t stats[4], bool f32, int parity) {
   const MergeParams mp = MergeParams::from_env();
   MergeStats        ms;
   HostCsr           S = merged_sweep_form(T, upper, mp, &ms);
   const unsigned    m = static_cast<unsigned>(T.nrows);
   if (sweep_kind() == 2) {
-    ws_host_emulate(S, upper, rhs, diag, x, stats, f32);
+    ws_host_emulate(S, upper, rhs, diag, x, stats, f32, parity);
     return;
   }
   std::vector<double> xg(2 * static_cast<std::size_t>(m), 0.0);
-  stream_host_emulate(S, upper, rhs, diag, xg.data(), stats, f32);
+  stream_host_emulate(S, upper, rhs, diag, xg.data(), stats, f32, parity);
   std::copy(xg.begin(), xg.begin() + m, x);
 }
 

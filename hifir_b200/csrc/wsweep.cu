@@ -202,8 +202,7 @@ void pack_warp_streams(const HostCsr &S, WsHost &H, unsigned nwarps, unsigned wi
     hd[2]        = (jump && level >= window) ? sentinel_of_level[level - window] : kWsNone;
     hd[3]        = level;
     last_level[warp] = static_cast<int>(level);
-    H.order.push_back(warp);
-    H.order.push_back(o);
+    ++H.nsegs;
     return hd;
   };
   for (unsigned p = 0; p < n;) {
@@ -268,7 +267,6 @@ void pack_warp_streams(const HostCsr &S, WsHost &H, unsigned nwarps, unsigned wi
   H.entries = S.col.size();
   H.depth   = depth;
   H.slices  = nslices;
-  H.nsegs   = H.order.size() / 2u;
   // ---- concatenate the private streams; descriptor = {offset (words / 4), segments, 0, 0, first sizes}
   std::size_t total = 0;
   for (unsigned w = 0; w < nwarps; ++w) total += ws[w].size();
@@ -284,11 +282,6 @@ void pack_warp_streams(const HostCsr &S, WsHost &H, unsigned nwarps, unsigned wi
     seg_base += d[1];
     H.max_segs  = std::max<std::size_t>(H.max_segs, seg_off[w].size());
     H.stream.insert(H.stream.end(), ws[w].begin(), ws[w].end());
-  }
-  // order entries: (warp, offset inside the private stream) -> absolute word offset
-  for (std::size_t k = 0; k < H.order.size(); k += 2) {
-    const unsigned w = H.order[k];
-    H.order[k + 1] += H.wdesc[static_cast<std::size_t>(w) * 8u] * 4u;
   }
   // segment sizes for the ring: wdesc[4..7] = sizes (in 16-byte units) of the first 4 segments, header
   // word 1 of segment k = size of segment k + stages (set by finalize_ring)
@@ -374,29 +367,86 @@ void ws_concat_ldu(const WsHost &L, const WsHost &U, WsHost &H) {
   }
 }
 
-// CPU emulation of the warp-stream sweep on the packed data (segments in creation order = level
-// order): lets tests check merge + packing without a GPU.  x has H.nslots entries.
-void ws_host_emulate_packed(const WsHost &H, bool upper, bool f32, const double *rhs, const double *diag, double *x) {
-  double acc[32];
-  for (std::size_t k = 0; k < H.order.size(); k += 2) {
-    const unsigned *hd    = H.stream.data() + H.order[k + 1];
-    const unsigned  width = hd[0] & 0xffu, z = (hd[0] >> 8) & 0xffu, flags = hd[0] >> 16;
+// The warps' streams of a packed plan in an order the device can run them: every warp in stream order, a
+// segment as soon as its sentinel, every slot it gathers and -- U part of a fused plan -- the L results it
+// reads as right-hand sides are published.  What a segment computes does not depend on the order in which
+// ready segments of different warps run, so this walk needs no creation order: it serves a plan copied
+// back from the device as well.  run(warp, header) is called for every segment that runs; pos (out):
+// segments run per warp.  Returns the number of segments that can never run (0: deadlock free).
+template <class F>
+std::size_t ws_walk_dataflow(const WsHost &H, bool fused, std::vector<std::size_t> &pos, F &&run) {
+  std::vector<char> ready[2] = {std::vector<char>(H.nslots, 0), std::vector<char>(fused ? H.nslots : 0u, 0)};
+  pos.assign(H.nwarps, 0);
+  std::size_t left = 0;
+  for (unsigned w = 0; w < H.nwarps; ++w) left += H.seg_off[w].size();
+  for (bool progress = true; progress && left;) {
+    progress = false;
+    for (unsigned w = 0; w < H.nwarps; ++w) {
+      const std::size_t base = static_cast<std::size_t>(H.wdesc[static_cast<std::size_t>(w) * 8u]) * 4u;
+      while (pos[w] < H.seg_off[w].size()) {
+        const unsigned *hd    = H.stream.data() + base + H.seg_off[w][pos[w]];
+        const unsigned  width = hd[0] & 0xffu, flags = hd[0] >> 16;
+        const bool      copy  = (flags & kSegCopy) != 0u, u2 = fused && (flags & kSegUpper) != 0u;
+        std::vector<char> &rd    = ready[u2 ? 1 : 0];
+        const unsigned     nrow  = copy ? width * 32u : 32u;
+        const unsigned *   codes = hd + kWsHdrWords, *slots = codes + nrow;
+        bool               ok    = hd[2] == kWsNone || rd[hd[2]];
+        if (ok && !copy) {
+          const unsigned *cols = hd + kWsHdrWords + 64u;
+          for (unsigned k = 0; k < width * 32u && ok; ++k)
+            if (cols[k] != kWsNone && !rd[cols[k]]) ok = false;
+        }
+        for (unsigned r = 0; u2 && r < nrow && ok; ++r)
+          if (slots[r] != kWsNone && !(codes[r] & kCodeZeroRhs) && !ready[0][codes[r] & kCodeSlotMask]) ok = false;
+        if (!ok) break;
+        run(w, hd);
+        if (copy || (flags & kSegLast))
+          for (unsigned r = 0; r < nrow; ++r)
+            if (slots[r] != kWsNone) rd[slots[r]] = 1;
+        ++pos[w];
+        --left;
+        progress = true;
+      }
+    }
+  }
+  return left;
+}
+
+// CPU emulation of the warp-stream sweep on the packed data, in the device's arithmetic order: per-lane fma
+// over the entry positions, the shfl_xor butterfly of the device, one accumulator per lane of every warp
+// (a slice of several segments carries it from one segment to the next).  x has H.nslots entries.
+// parity < 0: plain values.  parity 0 / 1: every published value goes through tag_set (its last mantissa
+// bit replaced by the parity) before any consumer reads it, as on the device, and the right-hand side of an
+// upper sweep -- on the device the L sweep's tagged result -- is tagged as well.  x2 (fused plan): the U
+// segments publish to x2 and read their right-hand side from the L segments' results in x.
+void ws_host_emulate_packed(const WsHost &H, bool upper, bool f32, const double *rhs, const double *diag, double *x,
+                            int parity, double *x2) {
+  const bool          fused = x2 != nullptr;
+  std::vector<double> accs(static_cast<std::size_t>(H.nwarps) * 32u, 0.0);
+  std::vector<std::size_t> pos;
+  auto pub = [&](double v) { return parity < 0 ? v : tag_set_host(v, static_cast<unsigned>(parity)); };
+  const std::size_t stuck = ws_walk_dataflow(H, fused, pos, [&](unsigned w, const unsigned *hd) {
+    const unsigned width = hd[0] & 0xffu, z = (hd[0] >> 8) & 0xffu, flags = hd[0] >> 16;
+    const bool     up    = fused ? (flags & kSegUpper) != 0u : upper;
+    double *       xw    = fused && up ? x2 : x;
+    const double * rh    = fused && up ? x : rhs;  // U part of a fused plan: the L segments' results
+    double *       acc   = accs.data() + static_cast<std::size_t>(w) * 32u;
     auto rhs_of = [&](unsigned code) {
       if (code & kCodeZeroRhs) return 0.0;
       const unsigned r = code & kCodeSlotMask;
-      return upper ? rhs[r] / diag[r] : rhs[r];
+      return up ? pub(rh[r]) / diag[r] : rh[r];
     };
     if (flags & kSegCopy) {
       const unsigned *codes = hd + kWsHdrWords, *slots = codes + width * 32u;
       for (unsigned r = 0; r < width * 32u; ++r)
-        if (slots[r] != kWsNone) x[slots[r]] = rhs_of(codes[r]);
-      continue;
+        if (slots[r] != kWsNone) xw[slots[r]] = pub(rhs_of(codes[r]));
+      return;
     }
     const unsigned *     codes = hd + kWsHdrWords, *slots = codes + 32u, *cols = slots + 32u;
     const unsigned char *vals  = reinterpret_cast<const unsigned char *>(cols + width * 32u);
     const unsigned       lpr   = 1u << z;
     for (unsigned j = 0; j < 32u; ++j) {
-      if (flags & kSegFirst) acc[j] = ((j & (lpr - 1u)) == 0u && codes[j] != kWsNone) ? rhs_of(codes[j]) : 0.0;
+      if (flags & kSegFirst) acc[j] = ((j & (lpr - 1u)) == 0u && slots[j] != kWsNone) ? rhs_of(codes[j]) : 0.0;
       for (unsigned u = 0; u < width; ++u) {
         const unsigned c = cols[u * 32u + j];
         if (c == kWsNone) continue;
@@ -408,7 +458,7 @@ void ws_host_emulate_packed(const WsHost &H, bool upper, bool f32, const double 
         } else {
           std::memcpy(&v, vals + static_cast<std::size_t>(u * 32u + j) * 8u, 8);
         }
-        acc[j] = std::fma(-v, x[c], acc[j]);
+        acc[j] = std::fma(-v, xw[c], acc[j]);
       }
     }
     if (flags & kSegLast) {
@@ -418,49 +468,18 @@ void ws_host_emulate_packed(const WsHost &H, bool upper, bool f32, const double 
         std::memcpy(acc, nw, sizeof(nw));
       }
       for (unsigned j = 0; j < 32u; j += lpr)
-        if (slots[j] != kWsNone) x[slots[j]] = acc[j];
+        if (slots[j] != kWsNone) xw[slots[j]] = pub(acc[j]);
     }
-  }
+  });
+  if (stuck) throw std::logic_error("warp-stream emulation: " + std::to_string(stuck) + " segments can never run");
 }
 
-// Dataflow check of a packed plan (host only): every warp walks its stream in order, a segment can
-// run when its sentinel and every slot it gathers are published.  Returns the number of segments
-// that can never run (0 = the static schedule is deadlock free).
+// Dataflow check of a packed plan (host only): returns the number of segments that can never run (0 = the
+// static schedule is deadlock free).
 std::size_t ws_check_schedule(const WsHost &H, bool f32, std::string *why) {
-  std::vector<char>        ready(H.nslots, 0);
-  std::vector<std::size_t> pos(H.nwarps, 0);
-  std::size_t              left = 0;
-  for (unsigned w = 0; w < H.nwarps; ++w) left += H.seg_off[w].size();
+  std::vector<std::size_t> pos;
   (void)f32;
-  for (bool progress = true; progress && left;) {
-    progress = false;
-    for (unsigned w = 0; w < H.nwarps; ++w) {
-      const std::size_t base = static_cast<std::size_t>(H.wdesc[static_cast<std::size_t>(w) * 8u]) * 4u;
-      while (pos[w] < H.seg_off[w].size()) {
-        const unsigned *hd    = H.stream.data() + base + H.seg_off[w][pos[w]];
-        const unsigned  width = hd[0] & 0xffu, flags = hd[0] >> 16;
-        bool            ok    = hd[2] == kWsNone || ready[hd[2]];
-        if (ok && !(flags & kSegCopy)) {
-          const unsigned *cols = hd + kWsHdrWords + 64u;
-          for (unsigned k = 0; k < width * 32u && ok; ++k)
-            if (cols[k] != kWsNone && !ready[cols[k]]) ok = false;
-        }
-        if (!ok) break;
-        if (flags & kSegCopy) {
-          const unsigned *slots = hd + kWsHdrWords + width * 32u;
-          for (unsigned r = 0; r < width * 32u; ++r)
-            if (slots[r] != kWsNone) ready[slots[r]] = 1;
-        } else if (flags & kSegLast) {
-          const unsigned *slots = hd + kWsHdrWords + 32u;
-          for (unsigned j = 0; j < 32u; ++j)
-            if (slots[j] != kWsNone) ready[slots[j]] = 1;
-        }
-        ++pos[w];
-        --left;
-        progress = true;
-      }
-    }
-  }
+  const std::size_t left = ws_walk_dataflow(H, false, pos, [](unsigned, const unsigned *) {});
   if (left && why) {
     for (unsigned w = 0; w < H.nwarps && why->size() < 400; ++w)
       if (pos[w] < H.seg_off[w].size()) {
@@ -1299,7 +1318,7 @@ void ws_debug_graph(const HostCsr &S, unsigned nsm, std::vector<unsigned> &dep_p
 }
 
 void ws_host_emulate(const HostCsr &S, bool upper, const double *rhs, const double *diag, double *x_by_row,
-                     std::size_t stats[4], bool f32) {
+                     std::size_t stats[4], bool f32, int parity) {
   const WsConfig cfg = ws_config();
   WsHost         H;
   pack_warp_streams(S, H, 148u * cfg.warps, static_cast<unsigned>(std::max(1, ws_env("HIFIR_B200_WS_WINDOW", 2))), f32,
@@ -1311,12 +1330,39 @@ void ws_host_emulate(const HostCsr &S, bool upper, const double *rhs, const doub
     if (stuck) throw std::logic_error("warp-stream schedule can not complete: " + std::to_string(stuck) + " segments stuck;" + why);
   }
   std::vector<double> x(H.nslots, 0.0);
-  ws_host_emulate_packed(H, upper, f32, rhs, diag, x.data());
+  ws_host_emulate_packed(H, upper, f32, rhs, diag, x.data(), parity);
   for (std::size_t r = 0; r < S.orig_rows; ++r) x_by_row[r] = x[H.slot_of[r]];
   stats[0] = H.slices;
   stats[1] = H.padded;
   stats[2] = H.stream.size() * 4u;
   stats[3] = H.depth;
+}
+
+// The emulation of a plan as the device holds it: wdesc and the segment stream copied back, every warp's
+// segment offsets recovered from the segment headers (a warp's segments are contiguous).  x (and x2 for a
+// fused plan): ws_nslots entries.
+void ws_emulate_device_plan(const SweepPlan &plan, const double *rhs, const double *diag, double *x, double *x2,
+                            unsigned parity) {
+  WsHost H;
+  H.nwarps = plan.ws_grid * plan.ws_warps;
+  H.nslots = plan.ws_nslots;
+  H.wdesc.resize(plan.ws_wdesc.n);
+  H.stream.resize(plan.ws_stream.n);
+  if (H.wdesc.size() != static_cast<std::size_t>(H.nwarps) * 8u) throw std::logic_error("warp-stream plan: descriptor size");
+  HIF_CUDA(cudaMemcpy(H.wdesc.data(), plan.ws_wdesc.p, H.wdesc.size() * 4u, cudaMemcpyDeviceToHost));
+  HIF_CUDA(cudaMemcpy(H.stream.data(), plan.ws_stream.p, H.stream.size() * 4u, cudaMemcpyDeviceToHost));
+  H.seg_off.assign(H.nwarps, {});
+  for (unsigned w = 0; w < H.nwarps; ++w) {
+    const std::size_t base = static_cast<std::size_t>(H.wdesc[static_cast<std::size_t>(w) * 8u]) * 4u;
+    std::size_t       off  = 0;
+    for (unsigned k = 0; k < H.wdesc[static_cast<std::size_t>(w) * 8u + 1u]; ++k) {
+      if (base + off + kWsHdrWords > H.stream.size()) throw std::logic_error("warp-stream plan: segment beyond the stream");
+      const unsigned hx = H.stream[base + off];
+      H.seg_off[w].push_back(static_cast<unsigned>(off));
+      off += seg_words(hx & 0xffu, ((hx >> 16) & kSegCopy) != 0u, plan.f32);
+    }
+  }
+  ws_host_emulate_packed(H, plan.upper, plan.f32, rhs, diag, x, static_cast<int>(parity), plan.fused ? x2 : nullptr);
 }
 
 namespace {
